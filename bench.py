@@ -567,6 +567,25 @@ def pcie_probe(c):
     return {"h2d_gbs": best["h2d"], "d2h_gbs": best["d2h"], "bytes": nbytes}
 
 
+DUMP_BYTES = 48 << 20   # --dump-outputs writes at most this much
+
+
+def dump_outputs(path, w, v, xr):
+    """Writes W [J][B][N], V_J [B][N] and the reconstruction [B][N] of one step as w.npy [J][P], v.npy [P] and xr.npy [P]
+    (float64): the values at P (signal, time) positions drawn once from a fixed seed, the same for every array and every
+    run of a workload, or at every position when the whole output fits in DUMP_BYTES."""
+    import numpy as np
+    import torch
+    levels, total = w.shape[0], v.numel()
+    keep = min(total, DUMP_BYTES // (8 * (levels + 2)))
+    idx = np.arange(total) if keep == total else np.sort(np.random.default_rng(1234).choice(total, keep, replace=False))
+    idx = torch.as_tensor(idx, device=v.device)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "w.npy"), w.reshape(levels, total).index_select(1, idx).cpu().numpy())
+    np.save(os.path.join(path, "v.npy"), v.reshape(total).index_select(0, idx).cpu().numpy())
+    np.save(os.path.join(path, "xr.npy"), xr.reshape(total).index_select(0, idx).cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -578,7 +597,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (a seeded sample of W, V_J and the "
+                         "reconstruction, float64) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload == "span"):
+        ap.error("--dump-outputs applies to the batch workloads of --impl b200")
     if args.impl == "reference":
         if args.workload == "span":
             args.workload = "single2p28_coif5_J10"
@@ -615,16 +641,16 @@ def main():
         sampler = ClockSampler(local_rank)
         if rank == 0:
             sampler.start()
-        d = extra_span(c, reps=max(args.steps, 3))
+        d = extra_span(c, reps=args.steps)
         clocks = sampler.stop() if rank == 0 else None
         if rank == 0:
-            line = {"metric": METRIC, "value": d["value"], "unit": UNIT, "n_gpus": world, "steps": max(args.steps, 3),
+            line = {"metric": METRIC, "value": d["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
                     "warmup": 1, "ms_per_step": d["ms_per_step"], "higher_is_better": True, "scaling": "strong",
                     "vs_baseline": None, "dtype": "f64", "data": "synthetic",
                     "config": {"workload": "single2p28_coif5_J10", "wavelet": "coif5", "signal_length": 1 << 28, "levels": 10,
                                "boundary": "PERIODIC", "sharding": f"contiguous spans of {d['span_per_rank']} samples, one halo "
                                "exchange per direction (NCCL send/recv)", "l2": d["l2"]},
-                    "roofline": d["roofline"], "cpu_baseline": None, "e2e": None, "gpu_launches": d["gpu_launches_per_step"] * max(args.steps, 3),
+                    "roofline": d["roofline"], "cpu_baseline": None, "e2e": None, "gpu_launches": d["gpu_launches_per_step"] * args.steps,
                     "clocks": clocks, "round_trip_max_abs_err": d["round_trip_max_abs_err"],
                     "halo_exchange_ms_per_step": d["halo_exchange_ms_per_step"],
                     "roofline_model_gsamples": d["roofline_model_gsamples"], "frac_of_roofline_model": d["frac_of_roofline_model"]}
@@ -668,6 +694,9 @@ def main():
     launches = eng.launch_count() - l0
     ms_step = c.max_over_ranks(e0.elapsed_time(e1)) / args.steps
     value = world * b * n / ms_step * 1e-6
+    if args.dump_outputs and rank == 0:
+        last = (args.steps - 1) % nsets
+        dump_outputs(args.dump_outputs, ws[last], vs[last], xr[last])
 
     # correctness guard inside the bench: the timed path must really invert (PERIODIC round trip)
     rt = float((xr[0] - xs[0]).abs().max())

@@ -13,8 +13,14 @@ N in {128, 129, 256} single level (ModwtPeriodicRoundTripTest.java:25-42), N = 5
 (MultiLevelModwtCorrectnessTest.java:27-72), N in {256, 500} PERIODIC + ZERO_PADDING
 (ParallelVsSequentialEquivalenceTest.java:18-49), plus SYMMETRIC and the SWT denoise of config #5's wavelet.
 
+What is stored: the arrays themselves come to 2 MB, so each one (input, W, V, reconstruction, denoised signal) is kept
+as the SHA-256 digest of its shape and float64 bytes, which pins every bit, plus a seeded sample of SAMPLE values with
+their flat positions, which shows what the values are when a digest stops matching.  The inputs are regenerated from
+their seeds by cases(); the SWT thresholds are stored whole.
+
 Run from the repo root:  python tests/golden/make_golden.py
 """
+import hashlib
 import os
 import sys
 
@@ -26,6 +32,38 @@ from oracle import cref, javarandom  # noqa: E402
 from oracle.wavelets import filters  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "modwt_golden.npz")
+SAMPLE = 32
+
+
+def digest(a):
+    """SHA-256 of the shape and the little-endian float64 bytes of `a`, as 32 uint8"""
+    a = np.ascontiguousarray(a, dtype="<f8")
+    return np.frombuffer(hashlib.sha256(repr(a.shape).encode() + a.tobytes()).digest(), dtype=np.uint8)
+
+
+def entry(name, a, rng):
+    """the stored form of the golden array `name`: {name/sha256, name/idx, name/val}"""
+    a = np.ascontiguousarray(a, dtype=np.float64)
+    idx = np.sort(rng.choice(a.size, min(a.size, SAMPLE), replace=False)).astype(np.int64)
+    return {name + "/sha256": digest(a), name + "/idx": idx, name + "/val": a.ravel()[idx]}
+
+
+def outputs(key, name, mode, levels, x):
+    """the oracle's arrays of one case, {w, v, xr} plus {denoise_soft1, denoise_soft0} for the swt_ cases, and those
+    cases' thresholds {thr_soft1, thr_soft0}"""
+    h, g, wid = filters(name)
+    w = np.empty((levels, x.shape[0], x.shape[1]))
+    v = np.empty_like(x)
+    xr = np.empty_like(x)
+    for i in range(x.shape[0]):
+        w[:, i, :], v[i] = cref.decompose(x[i], h, g, levels, mode)
+        xr[i] = cref.reconstruct(w[:, i, :], v[i], h, g, mode, wid)
+    arrays, thresholds = {"w": w, "v": v, "xr": xr}, {}
+    if key.startswith("swt_"):
+        for soft in (True, False):
+            arrays[f"denoise_soft{int(soft)}"], thresholds[f"thr_soft{int(soft)}"] = \
+                cref.swt_denoise(x[0], h, g, levels, mode, wid, -1.0, soft)
+    return arrays, thresholds
 
 
 def cases():
@@ -55,22 +93,14 @@ def cases():
 
 def main():
     blobs = {}
+    rng = np.random.default_rng(20240607)
     for key, name, mode, levels, x in cases():
-        h, g, wid = filters(name)
-        blobs[key + "/x"] = x
-        w = np.empty((levels, x.shape[0], x.shape[1]))
-        v = np.empty_like(x)
-        xr = np.empty_like(x)
-        for i in range(x.shape[0]):
-            wi, vi = cref.decompose(x[i], h, g, levels, mode)
-            w[:, i, :], v[i] = wi, vi
-            xr[i] = cref.reconstruct(wi, vi, h, g, mode, wid)
-        blobs[key + "/w"], blobs[key + "/v"], blobs[key + "/xr"] = w, v, xr
-        if key.startswith("swt_"):
-            for soft in (True, False):
-                den, thr = cref.swt_denoise(x[0], h, g, levels, mode, wid, -1.0, soft)
-                blobs[key + f"/denoise_soft{int(soft)}"] = den
-                blobs[key + f"/thr_soft{int(soft)}"] = np.array([thr])
+        arrays, thresholds = outputs(key, name, mode, levels, x)
+        blobs.update(entry(key + "/x", x, rng))
+        for k, a in arrays.items():
+            blobs.update(entry(f"{key}/{k}", a, rng))
+        for k, t in thresholds.items():
+            blobs[f"{key}/{k}"] = np.array([t])
     np.savez_compressed(OUT, **blobs)
     print(f"{OUT}: {len(blobs)} arrays, {os.path.getsize(OUT) / 1024:.0f} KiB")
 
