@@ -183,6 +183,23 @@ VW_API int vw_modwt_inverse(vw_ctx *ctx, const double *w, int64_t ldw, int64_t l
                      int32_t levels, int32_t mode, const vw_align *align, int32_t order, uint64_t detail_mask,
                      int32_t use_approx, double *xout, int64_t ldx, uint32_t flags);
 
+/* ---- single level over rows of different lengths -------------------------------------------------------------- */
+/* MODWTTransform.forwardBatch over rows of different lengths (CORE/modwt/MODWTTransform.java:486-515), i.e. one
+ * MODWTTransform.forward per row (:131-189): row b is x[offsets[b] .. offsets[b+1]), and its V and W are written at
+ * the same packed positions of v and w.  Same per-row rules as vw_modwt_forward with levels = 1 (any n >= 1, true
+ * multi-wrap when n < l).  offsets: a HOST array of batch + 1 values whatever the flags say, offsets[0] == 0, never
+ * decreasing (else VW_ELENGTH).  Rows are validated in index order like the reference's per-row loop: the lowest row
+ * that is empty (VW_EEMPTY) or, with VW_FLAG_CHECK_FINITE, holds a NaN / Inf (VW_ENONFINITE) fails the call, its index
+ * in vw_last_error.  One kernel launch however many rows; not capturable into a graph (VW_ESTATE). */
+VW_API int vw_modwt_forward_varlen(vw_ctx *ctx, const double *x, const int64_t *offsets, int64_t batch,
+                                   const double *hs, const double *gs, int32_t l, int32_t mode,
+                                   double *w, double *v, uint32_t flags);
+/* MODWTTransform.inverse per row (:203-299): pair-added products; PERIODIC / ZERO_PADDING use t+l, SYMMETRIC uses
+ * t-l (the rule inverseBatch applies when lengths differ).  Same packing as above; xout packed like w and v. */
+VW_API int vw_modwt_inverse_varlen(vw_ctx *ctx, const double *w, const double *v, const int64_t *offsets,
+                                   int64_t batch, const double *hs, const double *gs, int32_t l, int32_t mode,
+                                   double *xout, uint32_t flags);
+
 /* ---- thresholding / SWT denoise ------------------------------------------------------- */
 /* MutableMultiLevelMODWTResult.applyThreshold (CORE/modwt/MutableMultiLevelMODWTResult.java:83-118):
  * in place over `batch` rows of n; soft: |c|>t ? sign(c)*(|c|-t) : 0; hard: |c|<=t ? 0 : c.

@@ -247,7 +247,7 @@ public:
         const int64_t b = (int64_t)signals.size(), n = (int64_t)signals[0].size();
         bool same = true;
         for (const auto &s : signals) same = same && (int64_t)s.size() == n;
-        if (!same) { for (const auto &s : signals) out.push_back(forward(s)); return out; }
+        if (!same) return forwardMixed(signals);
         if (n == 0) throw InvalidSignalException("Signal cannot be empty", "VAL_006");
         std::vector<double> x((size_t)b * n), w((size_t)b * n), v((size_t)b * n);
         for (int64_t i = 0; i < b; i++) std::copy(signals[i].begin(), signals[i].end(), x.begin() + i * n);
@@ -261,6 +261,25 @@ public:
     }
 
 private:
+    // rows of different lengths: one packed vw_modwt_forward_varlen call; rows are validated in index order (the first
+    // empty or non-finite row throws, as forward() per row would)
+    std::vector<MODWTResult> forwardMixed(const std::vector<std::vector<double>> &signals) const {
+        const int64_t b = (int64_t)signals.size();
+        std::vector<int64_t> off((size_t)b + 1, 0);
+        for (int64_t i = 0; i < b; i++) off[i + 1] = off[i] + (int64_t)signals[i].size();
+        std::vector<double> x((size_t)off[b]), w((size_t)off[b]), v((size_t)off[b]);
+        for (int64_t i = 0; i < b; i++) std::copy(signals[i].begin(), signals[i].end(), x.begin() + off[i]);
+        Engine &e = Engine::get();
+        e.check(vw_modwt_forward_varlen(e.ctx(), x.data(), off.data(), b, hs_.data(), gs_.data(), (int)hs_.size(), (int)mode_,
+                                        w.data(), v.data(), VW_FLAG_CHECK_FINITE));
+        std::vector<MODWTResult> out;
+        out.reserve((size_t)b);
+        for (int64_t i = 0; i < b; i++)
+            out.emplace_back(std::vector<double>(v.begin() + off[i], v.begin() + off[i + 1]),
+                             std::vector<double>(w.begin() + off[i], w.begin() + off[i + 1]));
+        return out;
+    }
+
     Wavelet wavelet_;
     BoundaryMode mode_;
     std::vector<double> hs_, gs_;

@@ -96,6 +96,8 @@ public final class GpuMODWTOptimizer implements MODWTOptimizer, AutoCloseable {
     @Override
     public MODWTOptimizedResult[] forwardBatch(double[][] signals, Wavelet wavelet, BoundaryMode mode) {
         int b = signals.length, n = signals[0].length;
+        for (double[] s : signals)
+            if (s.length != n) return forwardBatchMixed(signals, wavelet, mode);
         double[] hs = scaled(wavelet.lowPassDecomposition()), gs = scaled(wavelet.highPassDecomposition());
         long bytes = (long) b * n * 8;
         PinnedArena pin = PinnedArena.current();      // pooled: cudaMallocHost per call would cost more than the transform
@@ -110,6 +112,37 @@ public final class GpuMODWTOptimizer implements MODWTOptimizer, AutoCloseable {
             MODWTOptimizedResult[] out = new MODWTOptimizedResult[b];
             for (int i = 0; i < b; i++)
                 out[i] = new Result(VwNative.copyOut(w, (long) i * n, n), VwNative.copyOut(v, (long) i * n, n));
+            return out;
+        } catch (Throwable t) {
+            throw VwNative.rethrow(t);
+        }
+    }
+
+    /** Rows of different lengths, each transformed at its own length: packed back to back and sent as ONE
+     *  vw_modwt_forward_varlen call (MODWTTransform.forwardBatch, MODWTTransform.java:486-515, runs forward per row). */
+    private MODWTOptimizedResult[] forwardBatchMixed(double[][] signals, Wavelet wavelet, BoundaryMode mode) {
+        int b = signals.length;
+        long[] off = new long[b + 1];
+        for (int i = 0; i < b; i++) off[i + 1] = off[i] + signals[i].length;
+        long total = off[b];
+        double[] hs = scaled(wavelet.lowPassDecomposition()), gs = scaled(wavelet.highPassDecomposition());
+        PinnedArena pin = PinnedArena.current();
+        pin.reset();
+        MemorySegment[] seg = pin.takeAll(total * 8, total * 8, total * 8);
+        MemorySegment x = seg[0], w = seg[1], v = seg[2];
+        try (Arena a = Arena.ofConfined()) {
+            for (int i = 0; i < b; i++)
+                MemorySegment.copy(signals[i], 0, x, ValueLayout.JAVA_DOUBLE, off[i] * 8, signals[i].length);
+            MemorySegment offseg = a.allocateFrom(ValueLayout.JAVA_LONG, off);
+            MemorySegment hseg = a.allocateFrom(ValueLayout.JAVA_DOUBLE, hs), gseg = a.allocateFrom(ValueLayout.JAVA_DOUBLE, gs);
+            int rc = (int) VwNative.vw_modwt_forward_varlen.invokeExact(ctx, x, offseg, (long) b, hseg, gseg, hs.length,
+                    modeOf(mode), w, v, VwNative.FLAG_CHECK_FINITE);
+            check(rc);
+            MODWTOptimizedResult[] out = new MODWTOptimizedResult[b];
+            for (int i = 0; i < b; i++) {
+                int n = signals[i].length;
+                out[i] = new Result(VwNative.copyOut(w, off[i], n), VwNative.copyOut(v, off[i], n));
+            }
             return out;
         } catch (Throwable t) {
             throw VwNative.rethrow(t);

@@ -55,6 +55,15 @@ public final class VwNative {
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, ADDRESS, JAVA_LONG, JAVA_LONG, JAVA_LONG,
                     ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS, JAVA_INT, JAVA_LONG, JAVA_INT, ADDRESS,
                     JAVA_LONG, JAVA_INT));
+    /** int vw_modwt_forward_varlen(ctx, x, const int64_t *offsets (host), batch, hs, gs, l, mode, w, v, flags) -- rows of
+     *  different lengths packed back to back (MODWTTransform.forwardBatch with mixed lengths) */
+    public static final MethodHandle vw_modwt_forward_varlen = h("vw_modwt_forward_varlen",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, ADDRESS,
+                    ADDRESS, JAVA_INT));
+    /** int vw_modwt_inverse_varlen(ctx, w, v, const int64_t *offsets (host), batch, hs, gs, l, mode, xout, flags) */
+    public static final MethodHandle vw_modwt_inverse_varlen = h("vw_modwt_inverse_varlen",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT,
+                    ADDRESS, JAVA_INT));
     /** int vw_swt_denoise(ctx, x, batch, n, ldx, hs, gs, l, levels, mode, align, order, threshold, soft, out, ldo,
      *  thresholds_out, flags) */
     public static final MethodHandle vw_swt_denoise = h("vw_swt_denoise",

@@ -93,6 +93,8 @@ SIGNATURES = {
                                    _i64, _u32]),
     "vw_modwt_inverse": (C.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _i64, _i64, _dp, _dp, _i32, _i32, _i32,
                                    C.POINTER(VwAlign), _i32, C.c_uint64, _i32, _vp, _i64, _u32]),
+    "vw_modwt_forward_varlen": (C.c_int, [_vp, _vp, C.POINTER(_i64), _i64, _dp, _dp, _i32, _i32, _vp, _vp, _u32]),
+    "vw_modwt_inverse_varlen": (C.c_int, [_vp, _vp, _vp, C.POINTER(_i64), _i64, _dp, _dp, _i32, _i32, _vp, _u32]),
     "vw_threshold": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _i32, _i32, _u32]),
     "vw_universal_threshold": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _u32]),
     "vw_swt_denoise": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _dp, _i32, _i32, _i32, C.POINTER(VwAlign), _i32,
@@ -446,6 +448,64 @@ class Engine:
                 gs.ctypes.data_as(_dp), hs.size, levels, int(mode), al, int(order), C.c_uint64(detail_mask),
                 int(bool(use_approx)), _vp(_ptr(res)), _ld(res), fl))
         return res[0] if one_d else res
+
+    @staticmethod
+    def _packed(a, what):
+        """1-D packed buffer: a contiguous float64 numpy array (pinned ones stay as they are) or CUDA tensor"""
+        if a is None:
+            raise NullPointerException(f"{what} cannot be null")
+        if _is_torch(a):
+            if a.dim() != 1:
+                raise IllegalArgumentException(f"packed {what} must be 1-D")
+            return a.contiguous()
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        if a.ndim != 1:
+            raise IllegalArgumentException(f"packed {what} must be 1-D")
+        return a
+
+    @staticmethod
+    def _offsets(offsets, size):
+        off = np.ascontiguousarray(offsets, dtype=np.int64)
+        if off.ndim != 1 or off.size < 2:
+            raise IllegalArgumentException("offsets must hold batch + 1 row boundaries")
+        if int(off[-1]) > size:
+            raise IllegalArgumentException(f"offsets end at {int(off[-1])}, beyond the packed buffer of {size} samples")
+        return off
+
+    def forward_varlen(self, x, offsets, hs, gs, mode, flags=0, w_out=None, v_out=None):
+        """Single-level forward of rows of different lengths in one launch: row b is x[offsets[b]:offsets[b+1]] of the
+        packed 1-D x; returns packed (W, V) with the same layout and residency (numpy, pinned numpy or CUDA tensor)."""
+        x = self._packed(x, "signal")
+        size = x.numel() if _is_torch(x) else x.size
+        off = self._offsets(offsets, size)
+        hs, gs = _fp(hs), _fp(gs)
+        if hs.size != gs.size:
+            raise IllegalArgumentException("low-pass and high-pass filters must have the same length")
+        w = w_out if w_out is not None else self._empty_like_rows(x, max(size, 1))
+        v = v_out if v_out is not None else self._empty_like_rows(x, max(size, 1))
+        with self._call_lock:
+            fl = self._bind_stream(x, w, v) | flags
+            self._check(self.lib.vw_modwt_forward_varlen(
+                self.ctx, _vp(_ptr(x)), off.ctypes.data_as(C.POINTER(_i64)), off.size - 1, hs.ctypes.data_as(_dp),
+                gs.ctypes.data_as(_dp), hs.size, int(mode), _vp(_ptr(w)), _vp(_ptr(v)), fl))
+        return w[:size], v[:size]
+
+    def inverse_varlen(self, w, v, offsets, hs, gs, mode, flags=0, out=None):
+        """Single-level inverse (MODWTTransform.inverse per row: pair-added, SYMMETRIC t-l, else t+l) of packed rows of
+        different lengths in one launch; returns the packed reconstruction."""
+        w, v = self._packed(w, "detail coefficients"), self._packed(v, "approximation coefficients")
+        size = w.numel() if _is_torch(w) else w.size
+        if (v.numel() if _is_torch(v) else v.size) != size:
+            raise IllegalArgumentException("approximation and detail buffers must have the same length")
+        off = self._offsets(offsets, size)
+        hs, gs = _fp(hs), _fp(gs)
+        res = out if out is not None else self._empty_like_rows(v, max(size, 1))
+        with self._call_lock:
+            fl = self._bind_stream(w, v, res) | flags
+            self._check(self.lib.vw_modwt_inverse_varlen(
+                self.ctx, _vp(_ptr(w)), _vp(_ptr(v)), off.ctypes.data_as(C.POINTER(_i64)), off.size - 1,
+                hs.ctypes.data_as(_dp), gs.ctypes.data_as(_dp), hs.size, int(mode), _vp(_ptr(res)), fl))
+        return res[:size]
 
     def threshold(self, coeffs, thresholds, soft, flags=0):
         """In place on `coeffs` ([B][N] or [N]); thresholds: scalar or per-row host values."""

@@ -177,6 +177,16 @@ int vw_launch_nonfinite_count(vw_ctx *ctx, const double *x, int64_t batch, int64
                               unsigned long long *count_dev);
 int vw_launch_energy(vw_ctx *ctx, const double *c, int64_t batch, int64_t n, int64_t ld, double *out_dev);
 
+// ---- single level over packed rows of different lengths (vw_varlen.cu) ---------------------------------------
+// off_dev: batch + 1 row offsets on the device (off_dev[b] - obase = start of row b in x / w / v, strictly increasing);
+// total = off_dev[batch] - obase packed samples.  Synthesis: SYMMETRIC takes t - k, the other modes t + k.
+int vw_launch_varlen_analysis(vw_ctx *ctx, const double *x, const int64_t *off_dev, int64_t batch, int64_t obase, int64_t total,
+                              const VwFilt &f, int l, int mode, double *w, double *v, bool exact);
+int vw_launch_varlen_synthesis(vw_ctx *ctx, const double *v, const double *w, const int64_t *off_dev, int64_t batch, int64_t obase,
+                               int64_t total, const VwFilt &f, int l, int mode, double *out, bool exact);
+// lowest index i < n with a[i] or b[i] (b may be null) NaN / Inf, atomically min-ed into *first_dev (preset to ~0)
+int vw_launch_first_nonfinite(vw_ctx *ctx, const double *a, const double *b, int64_t n, unsigned long long *first_dev);
+
 // ---- fused multi-level tile kernels (vw_fused.cu) ------------------------------------------
 // Return VW_OK when the fused path ran, VW_EUNSUPPORTED when the shape is not eligible (caller
 // falls back to the per-level kernels), anything else is an error.

@@ -401,18 +401,30 @@ int64_t pipe_rows(const vw_ctx *ctx, int64_t batch, int64_t n, int levels) {
     return (batch + chunks - 1) / chunks;
 }
 
-int forward_host_pipelined(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64_t ldx, const VwFilt &f, int l,
-                           int levels, int mode, double *w, int64_t ldw, int64_t lsw, double *vj, int64_t ldv, uint32_t flags,
-                           int64_t rows) {
+// runs chunk(c) for c = 0 .. nchunks-1, chunk c enqueued on pipeline stream c & 1 with scratch set c & 1; returns when
+// both streams have drained
+template <class Chunk>
+int run_pipelined(vw_ctx *ctx, int64_t nchunks, Chunk &&chunk) {
     int rc;
     if ((rc = pipe_streams(ctx))) return rc;
     if ((rc = vw_cuda_check(ctx, cudaStreamSynchronize(ctx->stream), "synchronize"))) return rc;
     PipeGuard guard(ctx);
-    int c = 0;
-    for (int64_t b0 = 0; b0 < batch; b0 += rows, c++) {
-        const int64_t rb = std::min(rows, batch - b0);
-        ctx->scratch_set = c & 1;
+    for (int64_t c = 0; c < nchunks; c++) {
+        ctx->scratch_set = (int)(c & 1);
         ctx->stream = ctx->pipe_stream[c & 1];
+        if ((rc = chunk(c))) return rc;
+    }
+    for (int i = 0; i < 2; i++)
+        if ((rc = vw_cuda_check(ctx, cudaStreamSynchronize(ctx->pipe_stream[i]), "pipeline synchronize"))) return rc;
+    return VW_OK;
+}
+
+int forward_host_pipelined(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64_t ldx, const VwFilt &f, int l,
+                           int levels, int mode, double *w, int64_t ldw, int64_t lsw, double *vj, int64_t ldv, uint32_t flags,
+                           int64_t rows) {
+    return run_pipelined(ctx, (batch + rows - 1) / rows, [&](int64_t c) -> int {
+        int rc;
+        const int64_t b0 = c * rows, rb = std::min(rows, batch - b0);
         void *px, *pw;
         const size_t bn = (size_t)rb * (size_t)n;
         if ((rc = vw_scratch(ctx, 2, (size_t)rows * (size_t)n * 8, &px))) return rc;
@@ -423,26 +435,17 @@ int forward_host_pipelined(vw_ctx *ctx, const double *x, int64_t batch, int64_t 
         if ((rc = forward_device(ctx, xd, rb, n, n, f, l, levels, mode, wd, n, (int64_t)bn, vd, n, flags))) return rc;
         for (int j = 0; j < levels; j++)
             if ((rc = copy_rows(ctx, w + (int64_t)j * lsw + b0 * ldw, ldw, wd + (size_t)j * bn, n, n, rb, cudaMemcpyDeviceToHost))) return rc;
-        if ((rc = copy_rows(ctx, vj + b0 * ldv, ldv, vd, n, n, rb, cudaMemcpyDeviceToHost))) return rc;
-    }
-    for (int i = 0; i < 2; i++)
-        if ((rc = vw_cuda_check(ctx, cudaStreamSynchronize(ctx->pipe_stream[i]), "pipeline synchronize"))) return rc;
-    return VW_OK;
+        return copy_rows(ctx, vj + b0 * ldv, ldv, vd, n, n, rb, cudaMemcpyDeviceToHost);
+    });
 }
 
 int inverse_host_pipelined(vw_ctx *ctx, const double *w, int64_t ldw, int64_t lsw, const double *vj, int64_t ldv,
                            int64_t batch, int64_t n, const VwFilt &f, int l, int levels, int mode, const vw_align *align,
                            int order, uint64_t detail_mask, int use_approx, double *xout, int64_t ldx, uint32_t flags,
                            int64_t rows) {
-    int rc;
-    if ((rc = pipe_streams(ctx))) return rc;
-    if ((rc = vw_cuda_check(ctx, cudaStreamSynchronize(ctx->stream), "synchronize"))) return rc;
-    PipeGuard guard(ctx);
-    int c = 0;
-    for (int64_t b0 = 0; b0 < batch; b0 += rows, c++) {
-        const int64_t rb = std::min(rows, batch - b0);
-        ctx->scratch_set = c & 1;
-        ctx->stream = ctx->pipe_stream[c & 1];
+    return run_pipelined(ctx, (batch + rows - 1) / rows, [&](int64_t c) -> int {
+        int rc;
+        const int64_t b0 = c * rows, rb = std::min(rows, batch - b0);
         void *px, *pw;
         const size_t bn = (size_t)rb * (size_t)n;
         if ((rc = vw_scratch(ctx, 2, (size_t)rows * (size_t)n * 8, &px))) return rc;
@@ -455,11 +458,8 @@ int inverse_host_pipelined(vw_ctx *ctx, const double *w, int64_t ldw, int64_t ls
             if ((rc = check_finite(ctx, wd, (int64_t)(levels + 1) * rb, n, n, "coefficients"))) return rc;
         if ((rc = inverse_device(ctx, wd, n, (int64_t)bn, vd, n, rb, n, f, l, levels, mode, align, order, detail_mask,
                                  use_approx, xd, n, flags, nullptr, 0, 0))) return rc;
-        if ((rc = copy_rows(ctx, xout + b0 * ldx, ldx, xd, n, n, rb, cudaMemcpyDeviceToHost))) return rc;
-    }
-    for (int i = 0; i < 2; i++)
-        if ((rc = vw_cuda_check(ctx, cudaStreamSynchronize(ctx->pipe_stream[i]), "pipeline synchronize"))) return rc;
-    return VW_OK;
+        return copy_rows(ctx, xout + b0 * ldx, ldx, xd, n, n, rb, cudaMemcpyDeviceToHost);
+    });
 }
 
 // Small host-buffer calls on PINNED memory skip the staging copies altogether: page-locked allocations are mapped into the
@@ -480,6 +480,93 @@ int check_signal_args(vw_ctx *ctx, const void *x, int64_t batch, int64_t n, int6
     if (n < 1) return vw_fail(ctx, VW_EEMPTY, "Signal cannot be empty");
     if (ld < n) return vw_fail(ctx, VW_ELENGTH, "row stride %lld shorter than signal length %lld", (long long)ld, (long long)n);
     return VW_OK;
+}
+
+// ---- packed rows of different lengths (vw_modwt_forward_varlen / vw_modwt_inverse_varlen) ---------------------------
+// offsets: HOST array of batch + 1 values, offsets[0] == 0, never decreasing.  *first_empty: the lowest empty row, or batch.
+int check_offsets(vw_ctx *ctx, const int64_t *off, int64_t batch, int64_t *first_empty) {
+    if (!off) return vw_fail(ctx, VW_ENULL, "offsets cannot be null");
+    if (batch < 1) return vw_fail(ctx, VW_ELENGTH, "signals must be non-null and non-empty (batch=%lld)", (long long)batch);
+    if (off[0] != 0) return vw_fail(ctx, VW_ELENGTH, "offsets[0] must be 0 (got %lld)", (long long)off[0]);
+    *first_empty = batch;
+    for (int64_t b = 0; b < batch; b++) {
+        if (off[b + 1] < off[b])
+            return vw_fail(ctx, VW_ELENGTH, "offsets decrease at row %lld (%lld -> %lld)", (long long)b, (long long)off[b],
+                           (long long)off[b + 1]);
+        if (off[b + 1] == off[b] && *first_empty == batch) *first_empty = b;
+    }
+    return VW_OK;
+}
+
+// row holding packed position p (empty rows hold none)
+int64_t row_of(const int64_t *off, int64_t batch, int64_t p) {
+    return (int64_t)(std::upper_bound(off, off + batch + 1, p) - off) - 1;
+}
+
+// lowest packed index i < n with a[i] or b[i] (b may be null) NaN / Inf, or -1.  Device pointers.
+int first_nonfinite(vw_ctx *ctx, const double *a, const double *b, int64_t n, int64_t *idx) {
+    *idx = -1;
+    if (n <= 0) return VW_OK;
+    void *slot = nullptr, *mb = nullptr;
+    int rc;
+    if ((rc = vw_scratch(ctx, 5, 64, &slot))) return rc;
+    if ((rc = pinned_mailbox(ctx, 64, &mb))) return rc;
+    if ((rc = vw_cuda_check(ctx, cudaMemsetAsync(slot, 0xff, 8, ctx->stream), "small copy"))) return rc;
+    if ((rc = vw_launch_first_nonfinite(ctx, a, b, n, (unsigned long long *)slot))) return rc;
+    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(mb, slot, 8, cudaMemcpyDeviceToHost, ctx->stream), "small copy"))) return rc;
+    if ((rc = vw_cuda_check(ctx, cudaStreamSynchronize(ctx->stream), "finite check"))) return rc;
+    const unsigned long long first = *(unsigned long long *)mb;
+    if (first != ~0ull) *idx = (int64_t)first;
+    return VW_OK;
+}
+
+// VW_ENONFINITE naming the row of the first bad packed index (chunk-local index q of a chunk starting at s0), if any
+int varlen_finite(vw_ctx *ctx, const double *a, const double *b, int64_t n, const int64_t *off, int64_t batch, int64_t s0,
+                  const char *what) {
+    int64_t q;
+    if (int rc = first_nonfinite(ctx, a, b, n, &q)) return rc;
+    if (q < 0) return VW_OK;
+    return vw_fail(ctx, VW_ENONFINITE, "row %lld: %s contain(s) non-finite values (NaN or Infinity)",
+                   (long long)row_of(off, batch, s0 + q), what);
+}
+
+// The reference's loop over rows (forwardBatch / inverseBatch with mixed lengths, one forward / inverse per row)
+// validates rows in index order and throws at the first bad one.  An empty row therefore fails the call, but only after
+// the rows before it were scanned for NaN / Inf.  a, b: the packed inputs (b may be null), host unless dev.
+int varlen_empty_row(vw_ctx *ctx, const double *a, const double *b, const int64_t *off, int64_t batch, int64_t empty, bool dev,
+                     bool check, const char *what) {
+    const int64_t lim = off[empty];
+    if (check && lim > 0) {
+        int rc;
+        if (!dev) {
+            void *p;
+            if ((rc = vw_scratch(ctx, 2, (size_t)lim * 8 * (b ? 2 : 1), &p))) return rc;
+            double *ad = (double *)p, *bd = b ? ad + lim : nullptr;
+            if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(ad, a, (size_t)lim * 8, cudaMemcpyHostToDevice, ctx->stream), "h2d"))) return rc;
+            if (b && (rc = vw_cuda_check(ctx, cudaMemcpyAsync(bd, b, (size_t)lim * 8, cudaMemcpyHostToDevice, ctx->stream), "h2d"))) return rc;
+            a = ad; b = bd;
+        }
+        if ((rc = varlen_finite(ctx, a, b, lim, off, batch, 0, what))) return rc;
+    }
+    return vw_fail(ctx, VW_EEMPTY, "row %lld: Signal cannot be empty", (long long)empty);
+}
+
+// row boundaries of the pipelined host path: about equal packed samples per chunk, cut between rows; a single cut
+// (one row holding nearly everything) means nothing to overlap
+std::vector<int64_t> varlen_chunks(const vw_ctx *ctx, const int64_t *off, int64_t batch) {
+    const int64_t total = off[batch];
+    const double bytes = (double)total * 8.0 * 3.0;
+    std::vector<int64_t> cut{0};
+    if (ctx->opt_pipe_min <= 0 || batch < 2 || bytes < (double)ctx->opt_pipe_min) return cut;
+    int64_t chunks = (int64_t)(bytes / (16.0 * 1048576.0));
+    chunks = std::max<int64_t>(2, std::min<int64_t>(std::min<int64_t>(chunks, std::max<int64_t>(ctx->opt_pipe_chunks, 2)), batch));
+    for (int64_t c = 1; c < chunks; c++) {
+        const int64_t b = (int64_t)(std::lower_bound(off, off + batch + 1, (int64_t)((double)total * c / chunks)) - off);
+        if (b > cut.back() && b < batch) cut.push_back(b);
+    }
+    cut.push_back(batch);
+    if (cut.size() < 3) cut.resize(1);
+    return cut;
 }
 
 }  // namespace vwshim
@@ -885,6 +972,143 @@ int vw_modwt_inverse(vw_ctx *ctx, const double *w, int64_t ldw, int64_t level_st
     if ((rc = inverse_device(ctx, wd, n, (int64_t)bn, vd, n, batch, n, f, l, levels, mode, align, order, detail_mask,
                              use_approx, xd, n, flags, nullptr, 0, 0))) return rc;
     if ((rc = copy_rows(ctx, xout, ldx, xd, n, n, batch, cudaMemcpyDeviceToHost))) return rc;
+    return finish(ctx, flags, true);
+}
+
+// MODWTTransform.forwardBatch / inverseBatch over rows of different lengths: one launch per direction (vw_varlen.cu)
+int vw_modwt_forward_varlen(vw_ctx *ctx, const double *x, const int64_t *offsets, int64_t batch, const double *hs,
+                            const double *gs, int32_t l, int32_t mode, double *w, double *v, uint32_t flags) {
+    if (!ctx) return VW_ENULL;
+    DeviceGuard g(ctx, "vw_modwt_forward_varlen");
+    if (int rc0 = no_capture(ctx, "vw_modwt_forward_varlen (host offsets)")) return rc0;
+    int rc;
+    if ((rc = check_mode(ctx, mode))) return rc;
+    if (!x) return vw_fail(ctx, VW_ENULL, "signal cannot be null");
+    if (!w || !v) return vw_fail(ctx, VW_ENULL, "output buffers cannot be null");
+    int64_t empty;
+    if ((rc = check_offsets(ctx, offsets, batch, &empty))) return rc;
+    VwFilt f;
+    if ((rc = load_filters(ctx, hs, gs, l, f))) return rc;
+    const bool dev = flags & VW_FLAG_DEVICE_PTRS, check = flags & VW_FLAG_CHECK_FINITE, exact = flags & VW_FLAG_BITEXACT;
+    if (empty < batch) return varlen_empty_row(ctx, x, nullptr, offsets, batch, empty, dev, check, "signal");
+    const int64_t total = offsets[batch];
+    void *po;
+    if ((rc = vw_scratch(ctx, 4, (size_t)(batch + 1) * 8, &po))) return rc;
+    int64_t *off_dev = (int64_t *)po;
+    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(off_dev, offsets, (size_t)(batch + 1) * 8, cudaMemcpyHostToDevice, ctx->stream),
+                            "offsets copy"))) return rc;
+    // rows [b0, b1) of the call, packed at xd / wd / vd
+    auto run = [&](const double *xd, double *wd, double *vd, int64_t b0, int64_t b1) -> int {
+        const int64_t s0 = offsets[b0], m = offsets[b1] - s0;
+        int r;
+        if (check && (r = varlen_finite(ctx, xd, nullptr, m, offsets, batch, s0, "signal"))) return r;
+        return vw_launch_varlen_analysis(ctx, xd, off_dev + b0, b1 - b0, s0, m, f, l, mode, wd, vd, exact);
+    };
+    if (dev) {
+        if ((rc = run(x, w, v, 0, batch))) return rc;
+        return finish(ctx, flags, false);
+    }
+    if (ctx->opt_zero_copy > 0 && (double)total * 24.0 <= (double)ctx->opt_zero_copy) {
+        const double *xa = (const double *)mapped_alias(x);
+        double *wa = xa ? (double *)mapped_alias(w) : nullptr, *va = wa ? (double *)mapped_alias(v) : nullptr;
+        if (xa && wa && va) {
+            if ((rc = run(xa, wa, va, 0, batch))) return rc;
+            return finish(ctx, flags, true);
+        }
+    }
+    const std::vector<int64_t> cut = varlen_chunks(ctx, offsets, batch);
+    if (cut.size() > 2) {
+        int64_t most = 0;
+        for (size_t c = 0; c + 1 < cut.size(); c++) most = std::max(most, offsets[cut[c + 1]] - offsets[cut[c]]);
+        return run_pipelined(ctx, (int64_t)cut.size() - 1, [&](int64_t c) -> int {
+            const int64_t b0 = cut[c], b1 = cut[c + 1], s0 = offsets[b0], m = offsets[b1] - s0;
+            void *px, *pw;
+            int r;
+            if ((r = vw_scratch(ctx, 2, (size_t)most * 8, &px))) return r;
+            if ((r = vw_scratch(ctx, 3, (size_t)most * 16, &pw))) return r;
+            double *xd = (double *)px, *wd = (double *)pw, *vd = wd + m;
+            if ((r = vw_cuda_check(ctx, cudaMemcpyAsync(xd, x + s0, (size_t)m * 8, cudaMemcpyHostToDevice, ctx->stream), "h2d"))) return r;
+            if ((r = run(xd, wd, vd, b0, b1))) return r;
+            if ((r = vw_cuda_check(ctx, cudaMemcpyAsync(w + s0, wd, (size_t)m * 8, cudaMemcpyDeviceToHost, ctx->stream), "d2h"))) return r;
+            return vw_cuda_check(ctx, cudaMemcpyAsync(v + s0, vd, (size_t)m * 8, cudaMemcpyDeviceToHost, ctx->stream), "d2h");
+        });
+    }
+    void *px, *pw;
+    if ((rc = vw_scratch(ctx, 2, (size_t)total * 8, &px))) return rc;
+    if ((rc = vw_scratch(ctx, 3, (size_t)total * 16, &pw))) return rc;
+    double *xd = (double *)px, *wd = (double *)pw, *vd = wd + total;
+    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(xd, x, (size_t)total * 8, cudaMemcpyHostToDevice, ctx->stream), "h2d"))) return rc;
+    if ((rc = run(xd, wd, vd, 0, batch))) return rc;
+    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(w, wd, (size_t)total * 8, cudaMemcpyDeviceToHost, ctx->stream), "d2h"))) return rc;
+    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(v, vd, (size_t)total * 8, cudaMemcpyDeviceToHost, ctx->stream), "d2h"))) return rc;
+    return finish(ctx, flags, true);
+}
+
+int vw_modwt_inverse_varlen(vw_ctx *ctx, const double *w, const double *v, const int64_t *offsets, int64_t batch,
+                            const double *hs, const double *gs, int32_t l, int32_t mode, double *xout, uint32_t flags) {
+    if (!ctx) return VW_ENULL;
+    DeviceGuard g(ctx, "vw_modwt_inverse_varlen");
+    if (int rc0 = no_capture(ctx, "vw_modwt_inverse_varlen (host offsets)")) return rc0;
+    int rc;
+    if ((rc = check_mode(ctx, mode))) return rc;
+    if (!w || !v) return vw_fail(ctx, VW_ENULL, "coefficient buffers cannot be null");
+    if (!xout) return vw_fail(ctx, VW_ENULL, "output buffer cannot be null");
+    int64_t empty;
+    if ((rc = check_offsets(ctx, offsets, batch, &empty))) return rc;
+    VwFilt f;
+    if ((rc = load_filters(ctx, hs, gs, l, f))) return rc;
+    const bool dev = flags & VW_FLAG_DEVICE_PTRS, check = flags & VW_FLAG_CHECK_FINITE, exact = flags & VW_FLAG_BITEXACT;
+    if (empty < batch) return varlen_empty_row(ctx, w, v, offsets, batch, empty, dev, check, "coefficients");
+    const int64_t total = offsets[batch];
+    void *po;
+    if ((rc = vw_scratch(ctx, 4, (size_t)(batch + 1) * 8, &po))) return rc;
+    int64_t *off_dev = (int64_t *)po;
+    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(off_dev, offsets, (size_t)(batch + 1) * 8, cudaMemcpyHostToDevice, ctx->stream),
+                            "offsets copy"))) return rc;
+    auto run = [&](const double *wd, const double *vd, double *xd, int64_t b0, int64_t b1) -> int {
+        const int64_t s0 = offsets[b0], m = offsets[b1] - s0;
+        int r;
+        if (check && (r = varlen_finite(ctx, wd, vd, m, offsets, batch, s0, "coefficients"))) return r;
+        return vw_launch_varlen_synthesis(ctx, vd, wd, off_dev + b0, b1 - b0, s0, m, f, l, mode, xd, exact);
+    };
+    if (dev) {
+        if ((rc = run(w, v, xout, 0, batch))) return rc;
+        return finish(ctx, flags, false);
+    }
+    if (ctx->opt_zero_copy > 0 && (double)total * 24.0 <= (double)ctx->opt_zero_copy) {
+        const double *wa = (const double *)mapped_alias(w);
+        const double *va = wa ? (const double *)mapped_alias(v) : nullptr;
+        double *xa = va ? (double *)mapped_alias(xout) : nullptr;
+        if (wa && va && xa) {
+            if ((rc = run(wa, va, xa, 0, batch))) return rc;
+            return finish(ctx, flags, true);
+        }
+    }
+    const std::vector<int64_t> cut = varlen_chunks(ctx, offsets, batch);
+    if (cut.size() > 2) {
+        int64_t most = 0;
+        for (size_t c = 0; c + 1 < cut.size(); c++) most = std::max(most, offsets[cut[c + 1]] - offsets[cut[c]]);
+        return run_pipelined(ctx, (int64_t)cut.size() - 1, [&](int64_t c) -> int {
+            const int64_t b0 = cut[c], b1 = cut[c + 1], s0 = offsets[b0], m = offsets[b1] - s0;
+            void *px, *pw;
+            int r;
+            if ((r = vw_scratch(ctx, 2, (size_t)most * 8, &px))) return r;
+            if ((r = vw_scratch(ctx, 3, (size_t)most * 16, &pw))) return r;
+            double *xd = (double *)px, *wd = (double *)pw, *vd = wd + m;
+            if ((r = vw_cuda_check(ctx, cudaMemcpyAsync(wd, w + s0, (size_t)m * 8, cudaMemcpyHostToDevice, ctx->stream), "h2d"))) return r;
+            if ((r = vw_cuda_check(ctx, cudaMemcpyAsync(vd, v + s0, (size_t)m * 8, cudaMemcpyHostToDevice, ctx->stream), "h2d"))) return r;
+            if ((r = run(wd, vd, xd, b0, b1))) return r;
+            return vw_cuda_check(ctx, cudaMemcpyAsync(xout + s0, xd, (size_t)m * 8, cudaMemcpyDeviceToHost, ctx->stream), "d2h");
+        });
+    }
+    void *px, *pw;
+    if ((rc = vw_scratch(ctx, 2, (size_t)total * 8, &px))) return rc;
+    if ((rc = vw_scratch(ctx, 3, (size_t)total * 16, &pw))) return rc;
+    double *xd = (double *)px, *wd = (double *)pw, *vd = wd + total;
+    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(wd, w, (size_t)total * 8, cudaMemcpyHostToDevice, ctx->stream), "h2d"))) return rc;
+    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(vd, v, (size_t)total * 8, cudaMemcpyHostToDevice, ctx->stream), "h2d"))) return rc;
+    if ((rc = run(wd, vd, xd, 0, batch))) return rc;
+    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(xout, xd, (size_t)total * 8, cudaMemcpyDeviceToHost, ctx->stream), "d2h"))) return rc;
     return finish(ctx, flags, true);
 }
 

@@ -311,7 +311,7 @@ class MODWTTransform:
                                    ORDER_PAIR, flags=self._flags)
 
     def forwardBatch(self, signals):
-        """:486-515 (+ :564-631).  Same-length signals run as one [B][N] launch; mixed lengths loop."""
+        """:486-515 (+ :564-631).  Same-length signals run as one [B][N] launch, mixed lengths as one packed launch."""
         if signals is None:
             raise NullPointerException("signals array cannot be null")
         if len(signals) == 0:
@@ -320,7 +320,7 @@ class MODWTTransform:
             raise NullPointerException("signal cannot be null")
         lengths = {_length(_as_signal(s)) for s in signals}
         if len(lengths) != 1:
-            return [self.forward(s) for s in signals]
+            return self._forward_mixed(signals)
         if _is_torch(signals):
             x = signals
         elif _is_torch(signals[0]):
@@ -344,7 +344,7 @@ class MODWTTransform:
         lengths = {r.getSignalLength() for r in results}
         n = results[0].getSignalLength()
         if len(lengths) != 1:
-            return [self.inverse(r) for r in results]
+            return self._inverse_mixed(results)
         optimized = len(results) >= 4 and n >= 64
         if not optimized:
             for r in results:
@@ -364,6 +364,50 @@ class MODWTTransform:
         out = self._eng().inverse(w.reshape(1, len(results), n), v, self._hrs, self._grs, self.boundaryMode.value,
                                   align, ORDER_PAIR, flags=self._flags)
         return [out[b] for b in range(len(results))]
+
+    # -- mixed lengths: one packed call per direction (vw_modwt_forward_varlen / vw_modwt_inverse_varlen) ----------------
+    @staticmethod
+    def _pack(rows):
+        """rows -> (packed buffer, offsets): torch.cat keeps CUDA tensors on the device, anything else packs on the host;
+        None when the rows mix residencies (those keep the per-row path)."""
+        offsets = np.zeros(len(rows) + 1, dtype=np.int64)
+        np.cumsum([int(r.shape[-1]) for r in rows], out=offsets[1:])
+        if all(_is_torch(r) and r.is_cuda for r in rows):
+            import torch
+            return torch.cat([r.reshape(-1) for r in rows]), offsets
+        if any(_is_torch(r) for r in rows):
+            return None, offsets
+        return np.concatenate([np.asarray(r, dtype=np.float64).reshape(-1) for r in rows]), offsets
+
+    def _forward_mixed(self, signals):
+        """forward() per row, as one launch.  Rows are checked in index order like the reference's loop: the first row
+        that is not 1-D raises here, after the rows before it ran (so an earlier empty or non-finite row still wins)."""
+        rows = [_as_signal(s) for s in signals]
+        bad = next((b for b, r in enumerate(rows) if r.ndim != 1), len(rows))
+        good = rows[:bad]
+        out = []
+        if good:
+            x, offsets = self._pack(good)
+            if x is None:
+                out = [self.forward(r) for r in good]
+            else:
+                w, v = self._eng().forward_varlen(x, offsets, self._hs, self._gs, self.boundaryMode.value,
+                                                  _native.FLAG_CHECK_FINITE | self._flags)
+                out = [MODWTResult(v[offsets[b]:offsets[b + 1]], w[offsets[b]:offsets[b + 1]], _validate=False)
+                       for b in range(len(good))]
+        if bad < len(rows):
+            raise IllegalArgumentException("forward takes one 1-D signal; use forwardBatch for [B][N]")
+        return out
+
+    def _inverse_mixed(self, results):
+        """inverse() per row (pair-added, SYMMETRIC t-l), as one launch; the lowest row with NaN / Inf raises."""
+        w, offsets = self._pack([r._d for r in results])
+        v, _ = self._pack([r._a for r in results])
+        if w is None or v is None or _is_torch(w) != _is_torch(v):
+            return [self.inverse(r) for r in results]
+        x = self._eng().inverse_varlen(w, v, offsets, self._hrs, self._grs, self.boundaryMode.value,
+                                       _native.FLAG_CHECK_FINITE | self._flags)
+        return [x[offsets[b]:offsets[b + 1]] for b in range(len(results))]
 
 
 class MultiLevelMODWTTransform:
