@@ -39,11 +39,12 @@ __device__ __forceinline__ unsigned long long key_of(double v) { return (unsigne
 // cand != nullptr: rows whose candidate buffers did not overflow read their candidates instead of the full row.
 template <int BITS>
 __global__ void __launch_bounds__(256)
-k_select_hist(const double *__restrict__ w, int64_t n, int64_t ld, const SelState *__restrict__ st, int shift,
+k_select_hist(const double *__restrict__ w, int64_t batch, int64_t n, int64_t ld, const SelState *__restrict__ st, int shift,
               unsigned int *__restrict__ hist /*[batch][2][1 << BITS]*/, const double *__restrict__ cand, unsigned int cap) {
     constexpr int BINS = 1 << BITS;
     __shared__ unsigned int sh[2][BINS];
-    const int64_t b = blockIdx.y;
+    const int64_t b = blockIdx.y + (int64_t)blockIdx.z * gridDim.y;   // batches beyond 32768 rows spill into grid.z
+    if (b >= batch) return;
     for (int i = threadIdx.x; i < 2 * BINS; i += blockDim.x) (&sh[0][0])[i] = 0;
     __syncthreads();
     const unsigned long long p0 = st[b].prefix[0], p1 = st[b].prefix[1];
@@ -121,9 +122,10 @@ __global__ void __launch_bounds__(256) k_select_pick(SelState *st, unsigned int 
 
 // compact the keys that share the decided high bits into the per-(row, which) candidate buffers
 __global__ void __launch_bounds__(256)
-k_select_collect(const double *__restrict__ w, int64_t n, int64_t ld, SelState *st, int decided_bits, double *cand,
-                 unsigned int cap) {
-    const int64_t b = blockIdx.y;
+k_select_collect(const double *__restrict__ w, int64_t batch, int64_t n, int64_t ld, SelState *st, int decided_bits,
+                 double *cand, unsigned int cap) {
+    const int64_t b = blockIdx.y + (int64_t)blockIdx.z * gridDim.y;
+    if (b >= batch) return;
     const unsigned long long p0 = st[b].prefix[0], p1 = st[b].prefix[1];
     const bool same = p0 == p1;
     const int hs = 64 - decided_bits;
@@ -193,19 +195,21 @@ static int select_median(vw_ctx *ctx, const double *w1, int64_t batch, int64_t n
     const int64_t capc = ((int64_t)ctx->sm_count * 16 + batch - 1) / batch;
     if (chunks > capc) chunks = capc;
     if (chunks < 1) chunks = 1;
-    const dim3 grid((unsigned)chunks, (unsigned)batch);
+    // one row per grid.y slot; gridDim.y stops at 65535, so rows beyond 32768 go to grid.z
+    const unsigned gy = (unsigned)(batch < 32768 ? batch : 32768);
+    const dim3 grid((unsigned)chunks, gy, (unsigned)((batch + gy - 1) / gy));
     // two 12-bit digits over the full rows: bits 63..52 (sign 0 + exponent), bits 51..40
     for (int shift = 64 - kBig; shift >= 64 - 2 * kBig; shift -= kBig) {
-        k_select_hist<kBig><<<grid, 256, 0, ctx->stream>>>(w1, n, ld, st, shift, hist, nullptr, 0u);
+        k_select_hist<kBig><<<grid, 256, 0, ctx->stream>>>(w1, batch, n, ld, st, shift, hist, nullptr, 0u);
         k_select_pick<kBig><<<(unsigned)(batch * 2), 256, 0, ctx->stream>>>(st, hist);
         ctx->launches += 2;
     }
-    k_select_collect<<<grid, 256, 0, ctx->stream>>>(w1, n, ld, st, 2 * kBig, cand, cap);
+    k_select_collect<<<grid, 256, 0, ctx->stream>>>(w1, batch, n, ld, st, 2 * kBig, cand, cap);
     k_select_mirror_count<<<nb, 128, 0, ctx->stream>>>(st, batch);
     ctx->launches += 2;
     // remaining 40 bits, 8 at a time, over the candidates (or the full row where they overflowed)
     for (int shift = 64 - 2 * kBig - 8; shift >= 0; shift -= 8) {
-        k_select_hist<8><<<grid, 256, 0, ctx->stream>>>(w1, n, ld, st, shift, hist, cand, cap);
+        k_select_hist<8><<<grid, 256, 0, ctx->stream>>>(w1, batch, n, ld, st, shift, hist, cand, cap);
         k_select_pick<8><<<(unsigned)(batch * 2), 256, 0, ctx->stream>>>(st, hist);
         ctx->launches += 2;
     }
