@@ -219,6 +219,31 @@ VW_API int vw_swt_denoise(vw_ctx *ctx, const double *x, int64_t batch, int64_t n
                    const double *gs, int32_t l, int32_t levels, int32_t mode, const vw_align *align, int32_t order,
                    double threshold, int32_t soft, double *out, int64_t ldo, double *thresholds_out, uint32_t flags);
 
+/* WaveletDenoiser's threshold selection methods (CORE/denoising/WaveletDenoiser.java:602-632, same order as ThresholdMethod). */
+typedef enum vw_threshold_method {
+    VW_THR_UNIVERSAL = 0,
+    VW_THR_SURE = 1,
+    VW_THR_MINIMAX = 2,
+    VW_THR_BAYES = 3,
+    VW_THR_FIXED = 4
+} vw_threshold_method;
+
+/* WaveletDenoiser over a [batch][n] batch in one call, every row on its own noise level.
+ * multilevel == 0: WaveletDenoiser.denoise / denoiseFixed (:111-145, :354-366): levels must be 1, any n >= 1 (multi-wrap
+ *   as vw_modwt_forward at one level), sigma = median(|W_1|) / 0.6745 unscaled; FIXED uses fixed_threshold.
+ * multilevel == 1: denoiseMultiLevel (:155-171, :183-231): sigma from each row's W_1, level j uses sigma / sqrt(2^j);
+ *   levels > 31 (MAX_SAFE_LEVEL_FOR_SCALING) is VW_ETOOLARGE, FIXED is VW_EUNSUPPORTED.
+ * UNIVERSAL s*sqrt(2 ln n); MINIMAX 0 (n <= 32), s*0.3936 + 0.1829*s*ln n (n <= 64), else s*(0.4745 + 0.1148 ln n);
+ * BAYES s^2 / sqrt(max(0, var(W_j) - s^2) + 1e-10); SURE the risk arg-min of vw_sure_threshold (levels * batch * n^2 <= 2^44,
+ * else VW_EUNSUPPORTED) capped at s*sqrt(2 ln n) -- each evaluated in the reference's operation order.  align / order are
+ * those of the matching reconstruct (MODWTTransform.inverse or MultiLevelMODWTTransform.reconstruct), as in vw_swt_denoise.
+ * The whole chain runs on the device with one synchronise at the end; the thresholds are applied as the synthesis loads W.
+ * thresholds_out: NULL or levels * batch HOST doubles, [level][row].  Not capturable into a graph. */
+VW_API int vw_wavelet_denoise(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64_t ldx, const double *hs,
+                              const double *gs, int32_t l, int32_t levels, int32_t mode, const vw_align *align, int32_t order,
+                              int32_t multilevel, int32_t method, double fixed_threshold, int32_t soft, double *out, int64_t ldo,
+                              double *thresholds_out, uint32_t flags);
+
 /* WaveletDenoiser.estimateNoiseSigma's order statistic (CORE/denoising/WaveletDenoiser.java:376-387,587-597): the exact
  * median of |c| per row (even count: mean of the two middle values).  sigma = median / 0.6745 stays on the host.
  * out: `batch` doubles on the HOST. */

@@ -69,6 +69,12 @@ public final class VwNative {
     public static final MethodHandle vw_swt_denoise = h("vw_swt_denoise",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT,
                     JAVA_INT, JAVA_INT, ADDRESS, JAVA_INT, JAVA_DOUBLE, JAVA_INT, ADDRESS, JAVA_LONG, ADDRESS, JAVA_INT));
+    /** int vw_wavelet_denoise(ctx, x, batch, n, ldx, hs, gs, l, levels, mode, align, order, multilevel, method,
+     *  fixed_threshold, soft, out, ldo, thresholds_out, flags) -- WaveletDenoiser over a batch, thresholds [level][row] */
+    public static final MethodHandle vw_wavelet_denoise = h("vw_wavelet_denoise",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT,
+                    JAVA_INT, JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_DOUBLE, JAVA_INT, ADDRESS, JAVA_LONG,
+                    ADDRESS, JAVA_INT));
     static final MethodHandle vw_threshold = h("vw_threshold",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, JAVA_LONG, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT));
     static final MethodHandle vw_universal_threshold = h("vw_universal_threshold",

@@ -25,6 +25,9 @@ FLAG_NO_SYNC = 1 << 4
 
 ORDER_SPLIT, ORDER_PAIR = 0, 1
 
+# vw_threshold_method: WaveletDenoiser.ThresholdMethod in declaration order
+THR_UNIVERSAL, THR_SURE, THR_MINIMAX, THR_BAYES, THR_FIXED = 0, 1, 2, 3, 4
+
 VW_OK = 0
 _STATUS = {
     1: (NullPointerException, None),
@@ -99,6 +102,8 @@ SIGNATURES = {
     "vw_universal_threshold": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _u32]),
     "vw_swt_denoise": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _dp, _i32, _i32, _i32, C.POINTER(VwAlign), _i32,
                                  C.c_double, _i32, _vp, _i64, _dp, _u32]),
+    "vw_wavelet_denoise": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _dp, _i32, _i32, _i32, C.POINTER(VwAlign), _i32,
+                                     _i32, _i32, C.c_double, _i32, _vp, _i64, _dp, _u32]),
     "vw_energy": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _u32]),
     "vw_median_abs": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _u32]),
     "vw_mean_variance": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _dp, _u32]),
@@ -545,6 +550,29 @@ class Engine:
                 int(levels), int(mode), al, int(order), float(threshold), int(bool(soft)), _vp(_ptr(res)), _ld(res),
                 thr.ctypes.data_as(_dp), fl))
         return (res[0], float(thr[0])) if one_d else (res, thr)
+
+    def wavelet_denoise(self, x, hs, gs, levels, mode, align=None, order=ORDER_SPLIT, multilevel=True,
+                        method=THR_UNIVERSAL, fixed_threshold=0.0, soft=True, flags=0):
+        """WaveletDenoiser over a [B][N] batch (or one [N] signal) in one call: x -> (denoised, thresholds [levels][B]),
+        both in x's residency (numpy, or CUDA tensors whose rows may have a stride ld > n)."""
+        x2, one_d = self._rows(x)
+        b, n = x2.shape
+        hs, gs = _fp(hs), _fp(gs)
+        res = self._empty_like_rows(x2, b, max(n, 1))
+        lev = max(int(levels), 1)
+        thr = np.empty((lev, max(b, 1)))
+        al = self._align_array(align, int(levels)) if align is not None else None
+        with self._call_lock:
+            fl = self._bind_stream(x2, res) | flags
+            self._check(self.lib.vw_wavelet_denoise(
+                self.ctx, _vp(_ptr(x2)), b, n, _ld(x2), hs.ctypes.data_as(_dp), gs.ctypes.data_as(_dp), hs.size,
+                int(levels), int(mode), al, int(order), int(bool(multilevel)), int(method), float(fixed_threshold),
+                int(bool(soft)), _vp(_ptr(res)), _ld(res), thr.ctypes.data_as(_dp), fl))
+        thr = thr[:, :b]
+        if _is_torch(x2):
+            import torch
+            thr = torch.as_tensor(thr, device=x2.device)
+        return (res[0], thr[:, 0]) if one_d else (res, thr)
 
     def median_abs(self, c, flags=0):
         """exact median(|c|) per row (WaveletDenoiser.estimateNoiseSigma's order statistic)"""

@@ -569,6 +569,7 @@ struct ColPairT {
                                           // themselves and ignore rows_per_chunk
     const double *thr; int thr_per_row, thr_soft;
     P c;                                  // the arithmetic core's coefficients (lattice, or the low-pass taps of a quadrature-mirror pair)
+    long long thr_lstride;                // synthesis: W_j reads thr[0], W_{j+1} reads thr[thr_lstride] (0: one table for both)
 };
 typedef ColPairT<ColLat> ColPair;
 
@@ -935,9 +936,11 @@ __global__ void __launch_bounds__(kCThreads, Core::CTAS) k_column_synthesis_pair
         const int nout = (int)left64;
         const int steps = __reduce_max_sync(mask, nout + lag);     // consumed own rows: the warp walks in step
         const long long pin0 = a.t0 + c2 + i0 * d2;                // position of consumed own row 0
-        const double lam = THR ? a.thr[a.thr_per_row ? b : 0] : 0.0;
-        const bool thr_nonneg = !(lam < 0.0);
-        auto thr = [&](double v) { return THR ? (thr_nonneg ? vw_threshold_nonneg(v, lam, a.thr_soft) : vw_threshold_value(v, lam, a.thr_soft)) : v; };
+        // the pair consumes two detail levels, each with its own threshold: lam1 for W_j, lam2 for W_{j+1}
+        const double lam1 = THR ? a.thr[a.thr_per_row ? b : 0] : 0.0;
+        const double lam2 = THR ? a.thr[a.thr_lstride + (a.thr_per_row ? b : 0)] : 0.0;
+        const bool thr_nonneg = !(lam1 < 0.0) && !(lam2 < 0.0);
+        auto thr = [&](double v, double lam) { return THR ? (thr_nonneg ? vw_threshold_nonneg(v, lam, a.thr_soft) : vw_threshold_value(v, lam, a.thr_soft)) : v; };
         // rows this lane (or, one step later, its partner) still needs; a short last chunk must not keep loading -- wrapped
         // or not -- while the longer chunks of its warp finish
         const int need = nout + lag + 1;
@@ -989,7 +992,7 @@ __global__ void __launch_bounds__(kCThreads, Core::CTAS) k_column_synthesis_pair
                 cp_async_wait<PD - 1>();
 #pragma unroll
                 for (int r = 0; r < R; r++) {
-                    const double cv = lds64(cur + r * kRow), cw2 = thr(lds64(cur + r * kRow + kStream)), cw1 = thr(lds64(cur + r * kRow + 2 * kStream));
+                    const double cv = lds64(cur + r * kRow), cw2 = thr(lds64(cur + r * kRow + kStream), lam2), cw1 = thr(lds64(cur + r * kRow + 2 * kStream), lam1);
                     *row_ptr(op, d2i, r) = core.row(a.c, r, rho, mask, cv, cw2, cw1);
                 }
             } else {
@@ -999,7 +1002,7 @@ __global__ void __launch_bounds__(kCThreads, Core::CTAS) k_column_synthesis_pair
                 cp_async_wait<PD - 1>();
 #pragma unroll
                 for (int r = 0; r < R; r++) {
-                    const double cv = lds64(cur + r * kRow), cw2 = thr(lds64(cur + r * kRow + kStream)), cw1 = thr(lds64(cur + r * kRow + 2 * kStream));
+                    const double cv = lds64(cur + r * kRow), cw2 = thr(lds64(cur + r * kRow + kStream), lam2), cw1 = thr(lds64(cur + r * kRow + 2 * kStream), lam1);
                     const double o = core.row(a.c, r, rho, mask, cv, cw2, cw1);
                     if (s0 + r >= lag && s0 + r < nout + lag) *row_ptr(op, d2i, r) = o;
                 }
@@ -1129,7 +1132,7 @@ static int launch_pair_analysis(vw_ctx *ctx, A &a, const double *x, int64_t ldx,
     a.x = x; a.ldx = ldx; a.wa = a.wb = nullptr; a.ldwa = a.ldwb = 0;
     a.o0 = v2; a.ldo0 = ldv2; a.o1 = w1; a.ldo1 = ldw1; a.o2 = w2; a.ldo2 = ldw2;
     a.n_in = n_in; a.t0 = t0; a.n_out = n_out; a.batch = batch; a.d = d; a.mode = mode;
-    a.thr = nullptr; a.thr_per_row = 0; a.thr_soft = 0;
+    a.thr = nullptr; a.thr_per_row = 0; a.thr_soft = 0; a.thr_lstride = 0;
     int per_sm = 0;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_column_analysis_pair<Core>, kCThreads, kRingBytes);
     dim3 grid;
@@ -1188,28 +1191,31 @@ static int launch_pair_synthesis(vw_ctx *ctx, A &a, int64_t n_out, int64_t d, in
 template <class A>
 static void fill_pair_synthesis(A &a, const double *v2, int64_t ldv2, const double *w2, int64_t ldw2, const double *w1, int64_t ldw1,
                                 double *out, int64_t ldo, int64_t n_in, int64_t t0, int64_t n_out, int64_t batch, int64_t d, int mode,
-                                const double *thr_dev, int thr_per_row, int thr_soft) {
+                                const double *thr_dev, int thr_per_row, int thr_soft, int64_t thr_lstride) {
     a.x = v2; a.ldx = ldv2; a.wa = w2; a.ldwa = ldw2; a.wb = w1; a.ldwb = ldw1;
     a.o0 = out; a.ldo0 = ldo; a.o1 = a.o2 = nullptr; a.ldo1 = a.ldo2 = 0;
     a.n_in = n_in; a.t0 = t0; a.n_out = n_out; a.batch = batch; a.d = d; a.mode = mode;
-    a.thr = thr_dev; a.thr_per_row = thr_per_row; a.thr_soft = thr_soft;
+    a.thr = thr_dev; a.thr_per_row = thr_per_row; a.thr_soft = thr_soft; a.thr_lstride = thr_lstride;
 }
 
 int vw_column_synthesis2(vw_ctx *ctx, const double *v2, int64_t ldv2, const double *w2, int64_t ldw2, const double *w1,
                          int64_t ldw1, double *out, int64_t ldo, int64_t n_in, int64_t t0, int64_t n_out, int64_t batch,
-                         const VwFilt &f, int l, int64_t d, int mode, const double *thr_dev, int thr_per_row, int thr_soft) {
+                         const VwFilt &f, int l, int64_t d, int mode, const double *thr_dev, int thr_per_row, int thr_soft,
+                         int64_t thr_lstride) {
     if (n_out < 1 || batch < 1 || !v2 || !w2 || !w1) return VW_EUNSUPPORTED;
     if (l == 30) {
         ColPair a;
         if (!pair_ok(ctx, f, l, d, mode, a.c)) return VW_EUNSUPPORTED;
-        fill_pair_synthesis(a, v2, ldv2, w2, ldw2, w1, ldw1, out, ldo, n_in, t0, n_out, batch, d, mode, thr_dev, thr_per_row, thr_soft);
+        fill_pair_synthesis(a, v2, ldv2, w2, ldw2, w1, ldw1, out, ldo, n_in, t0, n_out, batch, d, mode, thr_dev, thr_per_row, thr_soft,
+                            thr_lstride);
         return launch_pair_synthesis<LatSynCore<15>>(ctx, a, n_out, d, batch, thr_dev != nullptr);
     }
     // 16-20-tap quadrature-mirror pairs: direct form (their decimal tables fit no lattice)
     if (!dir_pair_ok(ctx, f, l, d, mode, 4)) return VW_EUNSUPPORTED;
     ColPairT<DirTaps> a;
     for (int k = 0; k < VW_LEAN_MAX_L; k++) a.c.h[k] = k < l ? f.h[k] : 0.0;
-    fill_pair_synthesis(a, v2, ldv2, w2, ldw2, w1, ldw1, out, ldo, n_in, t0, n_out, batch, d, mode, thr_dev, thr_per_row, thr_soft);
+    fill_pair_synthesis(a, v2, ldv2, w2, ldw2, w1, ldw1, out, ldo, n_in, t0, n_out, batch, d, mode, thr_dev, thr_per_row, thr_soft,
+                        thr_lstride);
     if (l == 16) return launch_pair_synthesis<DirSynCore<16>>(ctx, a, n_out, d, batch, thr_dev != nullptr);
     if (l == 18) return launch_pair_synthesis<DirSynCore<18>>(ctx, a, n_out, d, batch, thr_dev != nullptr);
     return launch_pair_synthesis<DirSynCore<20>>(ctx, a, n_out, d, batch, thr_dev != nullptr);

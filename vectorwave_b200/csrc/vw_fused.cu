@@ -265,6 +265,7 @@ struct InvArgs {
     const double *thr; int thr_per_row, thr_soft;
     long long off_v, off_w;   // stream offsets of an aligned single-level stage (SYMMETRIC sigma/tau); 0 otherwise
     VwFilt32 f;               // taps of a sigma = -1 stream arrive reversed
+    int thr_lstride;          // level lev of the group reads thr[lev * thr_lstride]; 0: one table for every level
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -576,7 +577,7 @@ __global__ void __launch_bounds__(kThreads, (L > 0 && L <= VW_LB4_MAXL) ? 4 : ((
         const double *cv = cur + (lev == top ? par_v : 0);
         const int in_ext = extent(lev);
         if (a.thr && have_w) {
-            threshold_tile(slot ? wb1 : wb0, in_ext + par_w, (P & 1) == 0, a.thr + (a.thr_per_row ? b : 0), a.thr_soft);
+            threshold_tile(slot ? wb1 : wb0, in_ext + par_w, (P & 1) == 0, a.thr + (a.thr_per_row ? b : 0) + lev * a.thr_lstride, a.thr_soft);
             __syncthreads();
         }
         const int ld2 = a.log2d0 + lev;
@@ -933,6 +934,7 @@ int vw_fused_inverse(vw_ctx *ctx, const VwFusedInv &p, const VwFilt &f) {
     const int64_t htot = ((hexact + 1) & ~1ll) + (aligned_stage ? 4 : 0);   // room for the parity sample of odd stream offsets
     if (hexact > p.n_in || htot > 12288) return VW_EUNSUPPORTED;
     if (p.first_level + p.nlevels - 1 > 30) return VW_EUNSUPPORTED;
+    if (p.thr_dev && p.thr_lstride * p.nlevels > 0x7fffffffll) return VW_EUNSUPPORTED;   // the kernels index levels in 32 bits
     const bool use_tma = (!p.v || aligned16(p.v)) && aligned16(p.w) && aligned16(p.out) && !(p.ldv & 1) && !(p.ldw & 1) &&
                          !(p.lsw & 1) && !(p.ldo & 1) && !(p.n_in & 1) && !(p.n_out & 1);
     const size_t smem_cap = ctx->smem_optin - 1024;
@@ -954,7 +956,7 @@ int vw_fused_inverse(vw_ctx *ctx, const VwFusedInv &p, const VwFilt &f) {
     a.detail_mask = p.detail_mask; a.n_in = p.n_in; a.n_out = p.n_out; a.batch = p.batch;
     a.tile = (int)tile; a.htot = (int)htot; a.nlev = p.nlevels; a.log2d0 = p.first_level - 1; a.mode = p.mode;
     a.tiles_per_row = (int)tiles_per_row; a.use_tma = use_tma; a.lrt = p.l;
-    a.thr = p.thr_dev; a.thr_per_row = p.thr_per_row; a.thr_soft = p.thr_soft;
+    a.thr = p.thr_dev; a.thr_per_row = p.thr_per_row; a.thr_soft = p.thr_soft; a.thr_lstride = p.thr_lstride;
     a.off_v = a.off_w = 0;
     bool rev_h = false, rev_g = false;
     if (aligned_stage) {

@@ -1,6 +1,7 @@
 // vw_internal.cuh -- shared declarations of the MODWT engine's translation units.
 #pragma once
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 
 #include <chrono>
@@ -157,7 +158,7 @@ int forward_device(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64
 int inverse_device(vw_ctx *ctx, const double *w, int64_t ldw, int64_t lsw, const double *vj, int64_t ldv, int64_t batch,
                    int64_t n, const VwFilt &f, int l, int levels, int mode, const vw_align *align, int order,
                    uint64_t detail_mask, int use_approx, double *xout, int64_t ldx, uint32_t flags, const double *thr_dev,
-                   int thr_per_row, int thr_soft);
+                   int thr_per_row, int thr_soft, int64_t thr_lstride);
 }  // namespace vwshim
 int vw_cuda_check(vw_ctx *ctx, cudaError_t e, const char *what);
 int vw_scratch(vw_ctx *ctx, int slot, size_t bytes, void **out);
@@ -210,6 +211,7 @@ struct VwFusedInv {
     int64_t tile;                            // 0 = choose here
     bool has_align = false;                  // single-level stage with a general (sigma, tau) alignment (any mode)
     vw_align align = {1, 0, 1, 0};
+    int64_t thr_lstride = 0;                 // level first+i reads thr_dev[i * thr_lstride]; 0: one table for every level
 };
 
 // Level schedule: which consecutive levels share one fused launch and with which tile, from a small cost model
@@ -241,7 +243,8 @@ int vw_column_analysis2(vw_ctx *ctx, const double *x, int64_t ldx, double *w1, i
                         int mode);
 int vw_column_synthesis2(vw_ctx *ctx, const double *v2, int64_t ldv2, const double *w2, int64_t ldw2, const double *w1,
                          int64_t ldw1, double *out, int64_t ldo, int64_t n_in, int64_t t0, int64_t n_out, int64_t batch,
-                         const VwFilt &f, int l, int64_t d, int mode, const double *thr_dev, int thr_per_row, int thr_soft);
+                         const VwFilt &f, int l, int64_t d, int mode, const double *thr_dev, int thr_per_row, int thr_soft,
+                         int64_t thr_lstride);
 
 // ---- exact order statistics (vw_select.cu) ---------------------------------------------------
 // median(|w1|) per row -> universal thresholds written to thr_dev[batch] (device).
@@ -254,3 +257,28 @@ int vw_launch_sure(vw_ctx *ctx, const double *c, int64_t batch, int64_t n, int64
                    double *thr_dev, double *risk_dev);
 int vw_launch_mean_variance(vw_ctx *ctx, const double *c, int64_t batch, int64_t n, int64_t ld, double *mean_dev,
                             double *var_dev);
+// WaveletDenoiser's threshold selectors (vw_select.cu: k_denoise_select) for `levels` x `batch` (level, row) pairs, in the
+// reference's arithmetic.  The scalars that depend on n and j alone come from the host, computed as denoising.py does.
+struct VwDenoiseSel {
+    const double *med;       // [batch] median(|W_1|) per row
+    const double *var;       // BAYES: [levels][batch] population variance of W_j per row
+    const double *sure;      // SURE: [levels][batch] arg-min of the risk scan
+    double *sig;             // non-null: write the per-(level, row) noise level s here instead of thresholds
+    double *thr;             // [levels][batch] thresholds
+    int64_t batch, n;
+    int levels, method, multilevel;
+    double root;             // sqrt(2 ln n)
+    double log_n;            // ln n
+    double minimax_c;        // 0.4745 + 0.1148 ln n
+    double fixed;            // FIXED
+    double level_scale[VW_MAX_LEVELS];   // sqrt(2^j), index j - 1
+};
+int vw_launch_denoise_select(vw_ctx *ctx, const VwDenoiseSel &a);
+// the selectors' scalars that depend on n and j alone, as denoising.py computes them (math.log, math.sqrt: the same libm)
+inline void vw_denoise_scalars(int64_t n, int levels, VwDenoiseSel &a) {
+    a.n = n;
+    a.log_n = log((double)n);
+    a.root = sqrt(2.0 * log((double)n));
+    a.minimax_c = 0.4745 + 0.1148 * a.log_n;
+    for (int j = 1; j <= VW_MAX_LEVELS; j++) a.level_scale[j - 1] = j <= levels ? sqrt((double)((int64_t)1 << j)) : 0.0;
+}

@@ -47,6 +47,7 @@ struct LeanInv {
     const double *thr; int thr_per_row, thr_soft;   // SWT denoise: threshold every W tile as it lands (nullptr: off)
     int ext[kMaxLev];     // input extent of each level of the group beyond the owned samples: Tt + ext[lev]
     double h[VW_LEAN_MAX_L], g[VW_LEAN_MAX_L];
+    int thr_lstride;         // level lev of the group reads thr[lev * thr_lstride]; 0: one table for every level
 };
 
 template <int L, bool QMF>
@@ -263,7 +264,7 @@ __global__ void __launch_bounds__(256, L <= 12 ? 3 : 2) k_lean_synthesis(const _
         if (a.thr) {
             // MutableMultiLevelMODWTResult.applyThresholdToArray (:97-118) on the landed tile: W is thresholded exactly once
             // on its way from HBM to the FMAs, the thresholded coefficients never exist in memory
-            const double lam = __ldg(a.thr + (a.thr_per_row ? b : 0));
+            const double lam = __ldg(a.thr + (a.thr_per_row ? b : 0) + lev * a.thr_lstride);
             const bool nonneg = !(lam < 0.0);
             double2 *w2 = reinterpret_cast<double2 *>(lean_smem + (2 + slot) * PB);
             const int n2 = (Tt + a.ext[lev]) >> 1;                  // extents are even
@@ -447,7 +448,7 @@ int vw_lean_inverse(vw_ctx *ctx, const VwFusedInv &p, const VwFilt32 &f, int64_t
     a.tile = (int)tile; a.htot = (int)htot; a.nlev = p.nlevels; a.log2d0 = p.first_level - 1; a.mode = p.mode;
     a.tiles_per_row = (int)tiles_per_row;
     a.pf_mask = (int)ctx->opt_l2pf;
-    a.thr = p.thr_dev; a.thr_per_row = p.thr_per_row; a.thr_soft = p.thr_soft;
+    a.thr = p.thr_dev; a.thr_per_row = p.thr_per_row; a.thr_soft = p.thr_soft; a.thr_lstride = p.thr_lstride;
     const int64_t d0 = 1ll << (p.first_level - 1);
     const int64_t dmax = d0 << (p.nlevels - 1);
     for (int i = 0; i < p.nlevels; i++) {

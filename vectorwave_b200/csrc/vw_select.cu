@@ -321,3 +321,50 @@ int vw_launch_sure(vw_ctx *ctx, const double *c, int64_t batch, int64_t n, int64
     ctx->launches += 2;
     return vw_cuda_check(ctx, cudaGetLastError(), "sure launch");
 }
+
+// ---- WaveletDenoiser's threshold selectors (CORE/denoising/WaveletDenoiser.java:391-552) ---------------------------------
+// One thread per (level, row).  The device does only correctly rounded operations in denoising.py's left-to-right order
+// (no contraction), so every threshold is the one the single-signal path computes on the host from the same medians,
+// variances and SURE arg-mins.
+namespace {
+__global__ void k_denoise_select(const VwDenoiseSel a) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t)a.levels * a.batch) return;
+    const int j = (int)(i / a.batch);                          // level j + 1
+    const int64_t b = i - (int64_t)j * a.batch;
+    const double sigma = __ddiv_rn(a.med[b], 0.6745);          // estimateNoiseSigma (:376-387)
+    const double s = a.multilevel ? __ddiv_rn(sigma, a.level_scale[j]) : sigma;   // sigma / sqrt(2^j) (:221)
+    if (a.sig) { a.sig[i] = s; return; }
+    double t;
+    switch (a.method) {
+        case VW_THR_UNIVERSAL: t = __dmul_rn(s, a.root); break;
+        case VW_THR_MINIMAX:                                   // :497-509
+            if (a.n <= 32) t = 0.0;
+            else if (a.n <= 64) t = __dadd_rn(__dmul_rn(s, 0.3936), __dmul_rn(__dmul_rn(0.1829, s), a.log_n));
+            else t = __dmul_rn(s, a.minimax_c);
+            break;
+        case VW_THR_BAYES: {                                   // :521-552; Python's max(0.0, d) keeps 0.0 unless d > 0
+            const double s2 = __dmul_rn(s, s);
+            const double d = __dsub_rn(a.var[i], s2);
+            const double sx = __dsqrt_rn(__dadd_rn(d > 0.0 ? d : 0.0, 1e-10));
+            t = __ddiv_rn(s2, sx);
+            break;
+        }
+        case VW_THR_SURE: {                                    // :465-469 capped at the universal threshold
+            const double u = __dmul_rn(s, a.root);
+            t = a.sure[i] > u ? u : a.sure[i];
+            break;
+        }
+        default: t = a.fixed; break;                           // VW_THR_FIXED
+    }
+    a.thr[i] = t;
+}
+}  // namespace
+
+int vw_launch_denoise_select(vw_ctx *ctx, const VwDenoiseSel &a) {
+    const int64_t count = (int64_t)a.levels * a.batch;
+    if (count <= 0) return VW_OK;
+    k_denoise_select<<<(unsigned)((count + 127) / 128), 128, 0, ctx->stream>>>(a);
+    ctx->launches++;
+    return vw_cuda_check(ctx, cudaGetLastError(), "denoise select launch");
+}

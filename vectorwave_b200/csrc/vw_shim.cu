@@ -273,8 +273,11 @@ int forward_device(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64
 int inverse_device(vw_ctx *ctx, const double *w, int64_t ldw, int64_t lsw, const double *vj, int64_t ldv,
                    int64_t batch, int64_t n, const VwFilt &f, int l, int levels, int mode, const vw_align *align,
                    int order, uint64_t detail_mask, int use_approx, double *xout, int64_t ldx, uint32_t flags,
-                   const double *thr_dev, int thr_per_row, int thr_soft) {
+                   const double *thr_dev, int thr_per_row, int thr_soft, int64_t thr_lstride) {
     const bool exact = flags & VW_FLAG_BITEXACT;
+    // thresholds of level j start at thr_dev + (j-1) * thr_lstride (stride 0: one table for every level); a stage gets
+    // the table of its first level, and a multi-level stage the stride to reach the others
+    auto thr_at = [&](int level) { return thr_dev ? thr_dev + (int64_t)(level - 1) * thr_lstride : nullptr; };
     // the fused synthesis kernels implement the {+1,0,+1,0} index rule (t + k*d) -- PERIODIC and ZERO_PADDING
     bool plain = true;
     if (align)
@@ -313,14 +316,16 @@ int inverse_device(vw_ctx *ctx, const double *w, int64_t ldw, int64_t lsw, const
             if ((rc = pick_out(g.first, out, ld_out))) return rc;
             VwFusedInv p{cur, ld_cur, w + (int64_t)(g.first - 1) * lsw, ldw, lsw,
                          (detail_mask >> (g.first - 1)) & ((g.nlev >= 64 ? ~0ull : ((1ull << g.nlev) - 1))),
-                         out, ld_out, batch, n, n, l, g.first, g.nlev, mode, thr_dev, thr_per_row, thr_soft, g.tile};
+                         out, ld_out, batch, n, n, l, g.first, g.nlev, mode, thr_at(g.first), thr_per_row, thr_soft, g.tile};
+            p.thr_lstride = thr_lstride;
             rc = vw_fused_inverse(ctx, p, f);
             if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
             if (rc == VW_OK) { cur = out; ld_cur = ld_out; pp ^= 1; }
         } else if (allow_fused && g.tile == -2 && g.nlev == 2 && cur && ((detail_mask >> (g.first - 1)) & 3ull) == 3ull) {
             if ((rc = pick_out(g.first, out, ld_out))) return rc;
             rc = vw_column_synthesis2(ctx, cur, ld_cur, w + (int64_t)g.first * lsw, ldw, w + (int64_t)(g.first - 1) * lsw, ldw, out,
-                                      ld_out, n, 0, n, batch, f, l, (int64_t)1 << (g.first - 1), mode, thr_dev, thr_per_row, thr_soft);
+                                      ld_out, n, 0, n, batch, f, l, (int64_t)1 << (g.first - 1), mode, thr_at(g.first), thr_per_row,
+                                      thr_soft, thr_lstride);
             if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
             if (rc == VW_OK) { cur = out; ld_cur = ld_out; pp ^= 1; }
         }
@@ -336,22 +341,22 @@ int inverse_device(vw_ctx *ctx, const double *w, int64_t ldw, int64_t lsw, const
                 const int col_min = allow_fused ? vw_column_min_level(ctx, l, false) : std::min(3, vw_column_min_level(ctx, l, false));
                 if (fast && level >= col_min && ctx->opt_poly != 0) {
                     rc = vw_column_synthesis(ctx, cur, ld_cur, wj, ldw, out, ld_out, n, 0, n, batch, f, l,
-                                             (int64_t)1 << (level - 1), mode, al, thr_dev, thr_per_row, thr_soft);
+                                             (int64_t)1 << (level - 1), mode, al, thr_at(level), thr_per_row, thr_soft);
                     if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
                 }
                 if (rc == VW_EUNSUPPORTED && fast && !allow_fused) {
                     VwFusedInv p{cur, ld_cur, w + (int64_t)(level - 1) * lsw, ldw, lsw, wj ? 1ull : 0ull, out, ld_out, batch, n, n,
-                                 l, level, 1, mode, thr_dev, thr_per_row, thr_soft, 0};
+                                 l, level, 1, mode, thr_at(level), thr_per_row, thr_soft, 0};
                     p.has_align = true;
                     p.align = al;
                     rc = vw_fused_inverse(ctx, p, f);
                     if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
                 }
                 if (rc == VW_EUNSUPPORTED) {
-                    // the per-level kernels have no threshold-on-load: threshold this level in place first (only
-                    // vw_swt_denoise passes thr_dev, and its W is engine scratch)
+                    // the per-level kernels have no threshold-on-load: threshold this level in place first (only the
+                    // denoisers pass thr_dev, and their W is engine scratch)
                     if (thr_dev && wj &&
-                        (rc = vw_launch_threshold(ctx, const_cast<double *>(wj), batch, n, ldw, thr_dev, thr_per_row, thr_soft)))
+                        (rc = vw_launch_threshold(ctx, const_cast<double *>(wj), batch, n, ldw, thr_at(level), thr_per_row, thr_soft)))
                         return rc;
                     rc = vw_launch_synthesis_level(ctx, cur, ld_cur, wj, ldw, out, ld_out, n, 0, n, batch, f, l,
                                                    (int64_t)1 << (level - 1), mode, al, order == VW_ORDER_PAIR, exact);
@@ -457,7 +462,7 @@ int inverse_host_pipelined(vw_ctx *ctx, const double *w, int64_t ldw, int64_t ls
         if (flags & VW_FLAG_CHECK_FINITE)
             if ((rc = check_finite(ctx, wd, (int64_t)(levels + 1) * rb, n, n, "coefficients"))) return rc;
         if ((rc = inverse_device(ctx, wd, n, (int64_t)bn, vd, n, rb, n, f, l, levels, mode, align, order, detail_mask,
-                                 use_approx, xd, n, flags, nullptr, 0, 0))) return rc;
+                                 use_approx, xd, n, flags, nullptr, 0, 0, 0))) return rc;
         return copy_rows(ctx, xout + b0 * ldx, ldx, xd, n, n, rb, cudaMemcpyDeviceToHost);
     });
 }
@@ -567,6 +572,41 @@ std::vector<int64_t> varlen_chunks(const vw_ctx *ctx, const int64_t *off, int64_
     cut.push_back(batch);
     if (cut.size() < 3) cut.resize(1);
     return cut;
+}
+
+// The denoisers' chain over one batch: stage x, decompose into scratch, let `select` put the thresholds on the device
+// (select(W, thr, per_row, level_stride); W is [levels][batch][n] scratch), reconstruct with them applied as the
+// synthesis loads W (MutableMultiLevelMODWTResult.applyThreshold :97-118 fused into the load; stages without a fused form
+// threshold their level in place just before consuming it), stage the result back.  The caller synchronises.
+template <class Select>
+int denoise_chain(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64_t ldx, const VwFilt &f, int l, int levels,
+                  int mode, const vw_align *align, int order, int soft, double *out, int64_t ldo, uint32_t flags, Select &&select) {
+    int rc;
+    const bool dev = flags & VW_FLAG_DEVICE_PTRS;
+    size_t bn = (size_t)batch * (size_t)n;
+    void *pw;
+    if ((rc = vw_scratch(ctx, 3, bn * 8 * (size_t)(levels + 1), &pw))) return rc;
+    double *wd = (double *)pw, *vd = wd + bn * (size_t)levels;
+    const double *xd = x;
+    double *od = out;
+    int64_t ldxd = ldx, ldod = ldo;
+    if (!dev) {
+        void *p;
+        if ((rc = vw_scratch(ctx, 2, bn * 8, &p))) return rc;
+        if ((rc = copy_rows(ctx, p, n, x, ldx, n, batch, cudaMemcpyHostToDevice))) return rc;
+        xd = (const double *)p; od = (double *)p; ldxd = n; ldod = n;
+    }
+    if (flags & VW_FLAG_CHECK_FINITE) if ((rc = check_finite(ctx, xd, batch, n, ldxd, "signal"))) return rc;
+    if ((rc = forward_device(ctx, xd, batch, n, ldxd, f, l, levels, mode, wd, n, (int64_t)bn, vd, n, flags))) return rc;
+    const double *thr = nullptr;
+    int per_row = 0;
+    int64_t lstride = 0;
+    if ((rc = select((const double *)wd, thr, per_row, lstride))) return rc;
+    uint64_t mask = levels >= 64 ? ~0ull : ((1ull << levels) - 1);
+    if ((rc = inverse_device(ctx, wd, n, (int64_t)bn, vd, n, batch, n, f, l, levels, mode, align, order, mask, 1, od,
+                             ldod, flags, thr, per_row, soft, lstride))) return rc;
+    if (!dev) if ((rc = copy_rows(ctx, out, ldo, od, n, n, batch, cudaMemcpyDeviceToHost))) return rc;
+    return VW_OK;
 }
 
 }  // namespace vwshim
@@ -937,7 +977,7 @@ int vw_modwt_inverse(vw_ctx *ctx, const double *w, int64_t ldw, int64_t level_st
                 if ((rc = check_finite(ctx, w + (int64_t)j * level_stride_w, batch, n, ldw, "detail coefficients"))) return rc;
         }
         if ((rc = inverse_device(ctx, w, ldw, level_stride_w, vj, ldv, batch, n, f, l, levels, mode, align, order,
-                                 detail_mask, use_approx, xout, ldx, flags, nullptr, 0, 0))) return rc;
+                                 detail_mask, use_approx, xout, ldx, flags, nullptr, 0, 0, 0))) return rc;
         return finish(ctx, flags, false);
     }
     if (ctx->opt_zero_copy > 0 && (double)batch * (double)n * 8.0 * (levels + 2) <= (double)ctx->opt_zero_copy &&
@@ -952,7 +992,7 @@ int vw_modwt_inverse(vw_ctx *ctx, const double *w, int64_t ldw, int64_t level_st
                     if ((rc = check_finite(ctx, wa + (int64_t)j * level_stride_w, batch, n, ldw, "detail coefficients"))) return rc;
             }
             if ((rc = inverse_device(ctx, wa, ldw, level_stride_w, va, ldv, batch, n, f, l, levels, mode, align, order, detail_mask,
-                                     use_approx, xa, ldx, flags, nullptr, 0, 0))) return rc;
+                                     use_approx, xa, ldx, flags, nullptr, 0, 0, 0))) return rc;
             return finish(ctx, flags, true);
         }
     }
@@ -970,7 +1010,7 @@ int vw_modwt_inverse(vw_ctx *ctx, const double *w, int64_t ldw, int64_t level_st
     if (flags & VW_FLAG_CHECK_FINITE)
         if ((rc = check_finite(ctx, wd, (int64_t)(levels + 1) * batch, n, n, "coefficients"))) return rc;
     if ((rc = inverse_device(ctx, wd, n, (int64_t)bn, vd, n, batch, n, f, l, levels, mode, align, order, detail_mask,
-                             use_approx, xd, n, flags, nullptr, 0, 0))) return rc;
+                             use_approx, xd, n, flags, nullptr, 0, 0, 0))) return rc;
     if ((rc = copy_rows(ctx, xout, ldx, xd, n, n, batch, cudaMemcpyDeviceToHost))) return rc;
     return finish(ctx, flags, true);
 }
@@ -1179,39 +1219,23 @@ int vw_swt_denoise(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64
     if ((rc = load_filters(ctx, hs, gs, l, f))) return rc;
     if ((rc = check_levels(ctx, n, l, levels))) return rc;
     if (order != VW_ORDER_SPLIT && order != VW_ORDER_PAIR) return vw_fail(ctx, VW_EINVAL, "unknown synthesis order %d", order);
-    const bool dev = flags & VW_FLAG_DEVICE_PTRS;
-    size_t bn = (size_t)batch * (size_t)n;
-    void *pw, *pt;
-    if ((rc = vw_scratch(ctx, 3, bn * 8 * (size_t)(levels + 1), &pw))) return rc;
+    void *pt;
     if ((rc = vw_scratch(ctx, 5, (size_t)batch * 8 + 64, &pt))) return rc;
-    double *wd = (double *)pw, *vd = wd + bn * (size_t)levels;
     double *thr_dev = (double *)((char *)pt + 64);
-    const double *xd = x;
-    double *od = out;
-    int64_t ldxd = ldx, ldod = ldo;
-    if (!dev) {
-        void *p;
-        if ((rc = vw_scratch(ctx, 2, bn * 8, &p))) return rc;
-        if ((rc = copy_rows(ctx, p, n, x, ldx, n, batch, cudaMemcpyHostToDevice))) return rc;
-        xd = (const double *)p; od = (double *)p; ldxd = n; ldod = n;
-    }
-    if (flags & VW_FLAG_CHECK_FINITE) if ((rc = check_finite(ctx, xd, batch, n, ldxd, "signal"))) return rc;
-    if ((rc = forward_device(ctx, xd, batch, n, ldxd, f, l, levels, mode, wd, n, (int64_t)bn, vd, n, flags))) return rc;
     int per_row = 0;
-    if (threshold < 0) {
-        per_row = 1;
-        if ((rc = vw_launch_universal_threshold(ctx, wd, batch, n, n, thr_dev))) return rc;
-    } else {
-        if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(thr_dev, &threshold, 8, cudaMemcpyHostToDevice, ctx->stream), "small copy"))) return rc;
-        cudaStreamSynchronize(ctx->stream);  // &threshold is a stack address
-    }
-    // reconstruct; the thresholding rides on the synthesis: fused stages threshold W while it sits in shared memory
-    // (MutableMultiLevelMODWTResult.applyThreshold :97-118 fused into the load), the other stages threshold their
-    // level in place just before consuming it
-    uint64_t mask = levels >= 64 ? ~0ull : ((1ull << levels) - 1);
-    if ((rc = inverse_device(ctx, wd, n, (int64_t)bn, vd, n, batch, n, f, l, levels, mode, align, order, mask, 1, od,
-                             ldod, flags, thr_dev, per_row, soft))) return rc;
-    if (!dev) if ((rc = copy_rows(ctx, out, ldo, od, n, n, batch, cudaMemcpyDeviceToHost))) return rc;
+    rc = denoise_chain(ctx, x, batch, n, ldx, f, l, levels, mode, align, order, soft, out, ldo, flags,
+                       [&](const double *wd, const double *&thr, int &thr_per_row, int64_t &lstride) -> int {
+        if (threshold < 0) {
+            per_row = 1;
+            if (int r = vw_launch_universal_threshold(ctx, wd, batch, n, n, thr_dev)) return r;
+        } else {
+            if (int r = vw_cuda_check(ctx, cudaMemcpyAsync(thr_dev, &threshold, 8, cudaMemcpyHostToDevice, ctx->stream), "small copy")) return r;
+            cudaStreamSynchronize(ctx->stream);  // &threshold is a stack address
+        }
+        thr = thr_dev; thr_per_row = per_row; lstride = 0;   // one table for every level
+        return VW_OK;
+    });
+    if (rc) return rc;
     if (thresholds_out) {
         if (per_row) {
             if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(thresholds_out, thr_dev, (size_t)batch * 8, cudaMemcpyDeviceToHost, ctx->stream), "small copy"))) return rc;
@@ -1219,6 +1243,67 @@ int vw_swt_denoise(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64
             for (int64_t b = 0; b < batch; b++) thresholds_out[b] = threshold;
         }
     }
+    return vw_cuda_check(ctx, cudaStreamSynchronize(ctx->stream), "denoise");
+}
+
+int vw_wavelet_denoise(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64_t ldx, const double *hs,
+                       const double *gs, int32_t l, int32_t levels, int32_t mode, const vw_align *align, int32_t order,
+                       int32_t multilevel, int32_t method, double fixed_threshold, int32_t soft, double *out, int64_t ldo,
+                       double *thresholds_out, uint32_t flags) {
+    if (!ctx) return VW_ENULL;
+    DeviceGuard g(ctx, "vw_wavelet_denoise");
+    if (int rc0 = no_capture(ctx, "vw_wavelet_denoise")) return rc0;
+    int rc;
+    if ((rc = check_mode(ctx, mode))) return rc;
+    if ((rc = check_signal_args(ctx, x, batch, n, ldx))) return rc;
+    if ((rc = check_signal_args(ctx, out, batch, n, ldo))) return rc;
+    VwFilt f;
+    if ((rc = load_filters(ctx, hs, gs, l, f))) return rc;
+    if (multilevel != 0 && multilevel != 1) return vw_fail(ctx, VW_EINVAL, "multilevel must be 0 or 1 (got %d)", multilevel);
+    if (method < VW_THR_UNIVERSAL || method > VW_THR_FIXED) return vw_fail(ctx, VW_EINVAL, "Unknown threshold selection method %d", method);
+    if (!multilevel && levels != 1) return vw_fail(ctx, VW_EINVAL, "single-level denoise takes levels = 1 (got %d)", levels);
+    if (multilevel && levels > 31)   // WaveletDenoiser.MAX_SAFE_LEVEL_FOR_SCALING (:57)
+        return vw_fail(ctx, VW_ETOOLARGE, "Decomposition level %d exceeds safe limit for scale-dependent thresholds", levels);
+    if ((rc = check_levels(ctx, n, l, levels))) return rc;
+    if (order != VW_ORDER_SPLIT && order != VW_ORDER_PAIR) return vw_fail(ctx, VW_EINVAL, "unknown synthesis order %d", order);
+    if (multilevel && method == VW_THR_FIXED)
+        return vw_fail(ctx, VW_EUNSUPPORTED, "Fixed threshold method requires explicit threshold value");
+    if (method == VW_THR_SURE && (double)levels * (double)batch * (double)n * (double)n > 17592186044416.0)
+        return vw_fail(ctx, VW_EUNSUPPORTED, "SURE scores n candidates against n coefficients (as the reference does): "
+                                             "levels * batch * n^2 = %.3g exceeds 2^44",
+                       (double)levels * (double)batch * (double)n * (double)n);
+    const int64_t jb = (int64_t)levels * batch;
+    // slot 5 past the finite check's 64 bytes: med [batch] | thr, sig, mean, var, sure, risk [levels][batch]
+    void *pt;
+    if ((rc = vw_scratch(ctx, 5, (size_t)(batch + 6 * jb) * 8 + 64, &pt))) return rc;
+    double *med = (double *)((char *)pt + 64), *thr_dev = med + batch, *sig = thr_dev + jb, *mean = sig + jb, *var = mean + jb,
+           *sure = var + jb, *risk = sure + jb;
+    VwDenoiseSel sel;
+    vw_denoise_scalars(n, levels, sel);
+    sel.med = med; sel.var = var; sel.sure = sure; sel.sig = nullptr; sel.thr = thr_dev;
+    sel.batch = batch; sel.levels = levels; sel.method = method; sel.multilevel = multilevel; sel.fixed = fixed_threshold;
+    rc = denoise_chain(ctx, x, batch, n, ldx, f, l, levels, mode, align, order, soft, out, ldo, flags,
+                       [&](const double *wd, const double *&thr, int &thr_per_row, int64_t &lstride) -> int {
+        // W is [levels][batch][n] contiguous: the per-(level, row) statistics are one launch over levels * batch rows
+        if (int r = vw_launch_median_abs(ctx, wd, batch, n, n, med)) return r;
+        if (method == VW_THR_BAYES)
+            if (int r = vw_launch_mean_variance(ctx, wd, jb, n, n, mean, var)) return r;
+        if (method == VW_THR_SURE) {
+            VwDenoiseSel s = sel;
+            s.sig = sig;   // the noise level each row's risk scan scores against
+            if (int r = vw_launch_denoise_select(ctx, s)) return r;
+            void *ws;
+            if (int r = vw_scratch(ctx, 4, vw_sure_workspace(jb, n), &ws)) return r;
+            if (int r = vw_launch_sure(ctx, wd, jb, n, n, sig, ws, sure, risk)) return r;
+        }
+        if (int r = vw_launch_denoise_select(ctx, sel)) return r;
+        thr = thr_dev; thr_per_row = 1; lstride = batch;
+        return VW_OK;
+    });
+    if (rc) return rc;
+    if (thresholds_out &&
+        (rc = vw_cuda_check(ctx, cudaMemcpyAsync(thresholds_out, thr_dev, (size_t)jb * 8, cudaMemcpyDeviceToHost, ctx->stream), "small copy")))
+        return rc;
     return vw_cuda_check(ctx, cudaStreamSynchronize(ctx->stream), "denoise");
 }
 
@@ -1468,7 +1553,7 @@ int vw_modwt_inverse_span(vw_ctx *ctx, const double *vin, const double *w, int64
     const bool column_first = nlevels == 1 && first_level >= vw_column_min_level(ctx, l, false) && ctx->opt_poly != 0;
     if (!exact && !(flags & VW_FLAG_NO_FUSE) && nlevels == 2 && first_level >= vw_column_min_level(ctx, l, false) && ctx->opt_poly != 0) {
         rc = vw_column_synthesis2(ctx, vin, 0, w + level_stride_w, 0, w, 0, vout, 0, n_in, 0, n_local, 1, f, l,
-                                  (int64_t)1 << (first_level - 1), VW_MODE_LINEAR, nullptr, 0, 0);
+                                  (int64_t)1 << (first_level - 1), VW_MODE_LINEAR, nullptr, 0, 0, 0);
         if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
     }
     if (rc == VW_EUNSUPPORTED && !exact && !(flags & VW_FLAG_NO_FUSE) && !column_first) {

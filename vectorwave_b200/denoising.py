@@ -18,8 +18,10 @@ import numpy as np
 
 from . import _native
 from ._native import ORDER_PAIR
-from .errors import ErrorCode, InvalidArgumentException, NativeEngineError
-from .modwt import MODWTTransform, MultiLevelMODWTTransform, _as_signal
+from ._native import _is_torch
+from .errors import (ErrorCode, IllegalArgumentException, InvalidArgumentException, InvalidSignalException,
+                     NativeEngineError, NullPointerException)
+from .modwt import MODWTTransform, MultiLevelMODWTTransform, _as_signal, multilevel_alignment
 from .wavelets import BoundaryMode, Daubechies
 
 
@@ -38,6 +40,9 @@ class ThresholdType(enum.Enum):     # :636-650
 
 MAX_SAFE_LEVEL_FOR_SCALING = 31     # :57
 BAYES_EPSILON = 1e-10               # :67
+
+_METHOD_CODE = {ThresholdMethod.UNIVERSAL: _native.THR_UNIVERSAL, ThresholdMethod.SURE: _native.THR_SURE,
+                ThresholdMethod.MINIMAX: _native.THR_MINIMAX, ThresholdMethod.BAYES: _native.THR_BAYES}
 
 
 class WaveletDenoiser:
@@ -127,3 +132,73 @@ class WaveletDenoiser:
             self.lastThresholds.append(thr)
             eng.threshold(d, thr, type == ThresholdType.SOFT)
         return t.reconstruct(res)
+
+    # ---- batches: [B][N] rows, each with its own noise level, in one engine call (vw_wavelet_denoise) ----------------
+    # Row b gets what the single-signal method gives signals[b]; the selectors run on the device in the same arithmetic.
+    @staticmethod
+    def _batch(signals):
+        if signals is None:
+            raise NullPointerException("signals cannot be null")
+        x = signals if _is_torch(signals) else np.asarray(signals, dtype=np.float64)
+        if x.ndim != 2:
+            raise IllegalArgumentException("batch methods take a [B][N] array of signals")
+        if x.shape[1] == 0:
+            raise InvalidSignalException("Signal cannot be empty", ErrorCode.VAL_EMPTY)
+        return x
+
+    @staticmethod
+    def _method_code(method):
+        if method == ThresholdMethod.FIXED:                         # :414-425
+            raise InvalidArgumentException("Fixed threshold method requires explicit threshold value",
+                                           ErrorCode.CFG_UNSUPPORTED_OPERATION)
+        if method not in _METHOD_CODE:
+            raise InvalidArgumentException("Unknown threshold selection method", ErrorCode.CFG_UNSUPPORTED_OPERATION)
+        return _METHOD_CODE[method]
+
+    def _denoise_batch(self, x, levels, multilevel, code, fixed, type, align, order):
+        t = MODWTTransform(self.wavelet, self.boundaryMode, self._engine)
+        try:
+            return t._eng().wavelet_denoise(x, t._hs, t._gs, levels, self.boundaryMode.value, align, order, multilevel,
+                                            code, fixed, type == ThresholdType.SOFT, _native.FLAG_CHECK_FINITE)
+        except NativeEngineError as e:                              # SURE: levels * batch * n^2 beyond the engine's bound
+            if code != _native.THR_SURE:
+                raise
+            raise InvalidArgumentException(str(e), ErrorCode.CFG_UNSUPPORTED_OPERATION) from e
+
+    def _single_align(self):
+        return [(-1, 0, -1, 0)] if self.boundaryMode == BoundaryMode.SYMMETRIC else None   # MODWTTransform.inverse
+
+    def denoiseBatch(self, signals, method, type=ThresholdType.SOFT):
+        """denoise() of every row of a [B][N] numpy array or CUDA tensor, returned as the same kind."""
+        x = self._batch(signals)
+        code = self._method_code(method)
+        return self._denoise_batch(x, 1, False, code, 0.0, type, self._single_align(), ORDER_PAIR)[0]
+
+    def denoiseFixedBatch(self, signals, threshold, type):
+        """denoiseFixed() of every row with the one given threshold."""
+        x = self._batch(signals)
+        return self._denoise_batch(x, 1, False, _native.THR_FIXED, float(threshold), type, self._single_align(),
+                                   ORDER_PAIR)[0]
+
+    def denoiseMultiLevelBatch(self, signals, levels, method, type):
+        """denoiseMultiLevel() of every row; lastThresholds becomes [B][J], row b as denoiseMultiLevel(signals[b])
+        leaves it."""
+        x = self._batch(signals)
+        t = MultiLevelMODWTTransform(self.wavelet, self.boundaryMode, self._engine)
+        n = int(x.shape[1])
+        max_levels = t._calculate_max_levels(n)
+        if levels is None:
+            levels = max_levels
+        if levels < 1 or levels > max_levels:
+            raise InvalidArgumentException(
+                f"Invalid number of decomposition levels: {levels} (maximum {max_levels} for signal length {n})",
+                ErrorCode.CFG_INVALID_DECOMPOSITION_LEVEL)
+        if levels > MAX_SAFE_LEVEL_FOR_SCALING:
+            raise InvalidArgumentException("Decomposition level exceeds safe limit for scale-dependent thresholds",
+                                           ErrorCode.VAL_TOO_LARGE)
+        code = self._method_code(method)
+        align, order = multilevel_alignment(self.wavelet, self.boundaryMode, levels)
+        out, thr = self._denoise_batch(x, levels, True, code, 0.0, type, align, order)
+        thr = thr.cpu().numpy() if _is_torch(thr) else thr
+        self.lastThresholds = np.ascontiguousarray(thr.T)
+        return out
