@@ -307,6 +307,34 @@ VW_API int vw_modwt_stream_level(vw_ctx *ctx, const double *vin, int64_t batch, 
                           const double *hs, const double *gs, int32_t l, int32_t level, double *w, int64_t ldw,
                           double *v, int64_t ldv, uint32_t flags);
 
+/* ---- stream state on the device: the whole block cascade of BatchStreamingMODWT per call ------------------------- */
+/* BatchStreamingMODWT.processSingleLevel / processMultiLevel / flushSingleLevel / flushMultiLevel
+ * (EXT/extensions/modwt/BatchStreamingMODWT.java:55-276) with every level's left history kept in HBM by the handle:
+ * level j keeps the last (l-1)*2^(j-1) samples of its own input.
+ *  - create: mode ZERO_PADDING or SYMMETRIC (PERIODIC streaming is stateless: use vw_modwt_forward; anything else is
+ *    VW_EBOUNDARY), levels 1..30 (else VW_ELEVEL).  The handle copies the taps and belongs to ctx's device.
+ *  - process: x [batch][n] (row stride ldx) -> w [levels][batch][n] (strides level_stride_w, ldw), v = V_J [batch][n].
+ *    Any n >= 1 (the history carries the left context).  The first block after create / reset, and a block whose batch
+ *    differs from the previous one (:306-320), start the stream: level j's history is zeros, or for SYMMETRIC the
+ *    half-sample mirror of level j's own first input (multi-wrap when n is shorter than the history, :326-334).  After
+ *    every level the history becomes the last (l-1)*2^(j-1) samples of [history | input] (:336-350).
+ *  - flush: the cascade over a tail of tail_length samples built from the level-1 history (zeros, or that history
+ *    reversed for SYMMETRIC, :358-372); the histories are not advanced (:205-222,252-274).  VW_ESTATE before any block,
+ *    VW_ELENGTH for tail_length > l - 1, VW_EEMPTY for tail_length < 1.  Outputs [levels][batch][tail_length].
+ *  - reset: back to "no block seen" (no device work).
+ * Pointers are host pointers (staged) unless VW_FLAG_DEVICE_PTRS; VW_FLAG_CHECK_FINITE checks x, VW_FLAG_BITEXACT gives
+ * the reference's separate roundings, VW_FLAG_NO_FUSE forces the per-level kernels.  A failed call leaves the state as
+ * it was.  Not capturable into a graph (VW_ESTATE): every call advances the state on the host side. */
+typedef struct vw_stream_state vw_stream_state;
+VW_API int vw_stream_create(vw_ctx *ctx, const double *hs, const double *gs, int32_t l, int32_t levels, int32_t mode,
+                            vw_stream_state **out);
+VW_API int vw_stream_destroy(vw_ctx *ctx, vw_stream_state *st);
+VW_API int vw_stream_process(vw_ctx *ctx, vw_stream_state *st, const double *x, int64_t batch, int64_t n, int64_t ldx,
+                             double *w, int64_t ldw, int64_t level_stride_w, double *v, int64_t ldv, uint32_t flags);
+VW_API int vw_stream_flush(vw_ctx *ctx, vw_stream_state *st, int64_t tail_length, double *w, int64_t ldw,
+                           int64_t level_stride_w, double *v, int64_t ldv, uint32_t flags);
+VW_API int vw_stream_reset(vw_stream_state *st);
+
 /* ---- span-sharded long signals, whole cascade per rank (up-front halo schedule) ---------------------------- */
 /* The halo a rank needs is tiny next to its span ((l-1)*(2^levels-1) samples), so it is exchanged ONCE per direction:
  * before the analysis every rank receives the last `lead` samples of its left neighbour's x; before the synthesis the

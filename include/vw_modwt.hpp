@@ -545,6 +545,83 @@ struct BatchMODWT {
     }
 };
 
+// ---- BatchStreamingMODWT (EXT/extensions/modwt/BatchStreamingMODWT.java:55-276) ----------------------------------------
+// ZERO_PADDING / SYMMETRIC blocks continue each other through histories the engine keeps in HBM (vw_stream_state, owned
+// here: RAII); PERIODIC has no state and transforms each block on its own (:62-64,113-115).
+struct IllegalStateException : std::logic_error { using std::logic_error::logic_error; };
+struct UnsupportedOperationException : std::logic_error { using std::logic_error::logic_error; };
+
+class BatchStreamingMODWT {
+public:
+    struct SingleLevelResult { std::vector<double> approx /*[B][N]*/, detail /*[B][N]*/; int batch, n; };
+    using MultiLevelResult = BatchMODWT::MultiLevelResult;
+
+    BatchStreamingMODWT(const Wavelet &w, BoundaryMode mode, int levels = 1)
+        : mode_(mode), levels_(levels), hs_(detail::scaled(w.lowPassDecomposition())), gs_(detail::scaled(w.highPassDecomposition())) {
+        if (levels < 1) throw IllegalArgumentException("levels must be >= 1");
+        detail::require_mode(mode);
+    }
+    ~BatchStreamingMODWT() { if (st_) vw_stream_destroy(Engine::get().ctx(), st_); }
+    BatchStreamingMODWT(const BatchStreamingMODWT &) = delete;
+    BatchStreamingMODWT &operator=(const BatchStreamingMODWT &) = delete;
+
+    SingleLevelResult processSingleLevel(const std::vector<std::vector<double>> &signals) {   // :55-103
+        if (levels_ != 1) throw IllegalStateException("This instance is configured for levels=" + std::to_string(levels_) + ", expected=1");
+        MultiLevelResult r = processMultiLevel(signals);
+        return {std::move(r.finalApprox), std::move(r.detailPerLevel), r.batch, r.n};
+    }
+    MultiLevelResult processMultiLevel(const std::vector<std::vector<double>> &signals) {    // :111-163
+        if (signals.empty()) throw IllegalArgumentException("signals must be non-null and non-empty");
+        const int64_t b = (int64_t)signals.size(), n = (int64_t)signals[0].size();
+        if (n == 0) throw IllegalArgumentException("signal length must be > 0");
+        for (const auto &s : signals) if ((int64_t)s.size() != n) throw IllegalArgumentException("all signals must be non-null and same length");
+        std::vector<double> x((size_t)b * n);
+        for (int64_t i = 0; i < b; i++) std::copy(signals[i].begin(), signals[i].end(), x.begin() + i * n);
+        MultiLevelResult r{std::vector<double>((size_t)levels_ * b * n), std::vector<double>((size_t)b * n), levels_, (int)b, (int)n};
+        Engine &e = Engine::get();
+        if (mode_ == BoundaryMode::PERIODIC) {
+            e.check(vw_modwt_forward(e.ctx(), x.data(), b, n, n, hs_.data(), gs_.data(), (int)hs_.size(), levels_, VW_PERIODIC,
+                                     r.detailPerLevel.data(), n, b * n, r.finalApprox.data(), n, 0));
+            return r;
+        }
+        if (!st_) e.check(vw_stream_create(e.ctx(), hs_.data(), gs_.data(), (int)hs_.size(), levels_, (int)mode_, &st_));
+        e.check(vw_stream_process(e.ctx(), st_, x.data(), b, n, n, r.detailPerLevel.data(), n, b * n, r.finalApprox.data(), n, 0));
+        batch_ = (int)b;
+        return r;
+    }
+    SingleLevelResult flushSingleLevel(int tailLength) {   // :183-222
+        if (levels_ != 1) throw IllegalStateException("This instance is configured for levels=" + std::to_string(levels_) + ", expected=1");
+        MultiLevelResult r = flushMultiLevel(tailLength);
+        return {std::move(r.finalApprox), std::move(r.detailPerLevel), r.batch, r.n};
+    }
+    MultiLevelResult flushMultiLevel(int tailLength) {      // :231-276; the histories are not advanced
+        if (mode_ == BoundaryMode::PERIODIC) throw UnsupportedOperationException("Flush is only applicable to ZERO_PADDING/SYMMETRIC");
+        if (tailLength <= 0) return {{}, {}, levels_, 0, 0};
+        if (!st_ || batch_ == 0) throw IllegalStateException("No prior blocks processed; cannot flush");
+        if (tailLength > getMinFlushTailLength())
+            throw IllegalArgumentException("tailLength (" + std::to_string(tailLength) + ") exceeds maximum allowed across levels (" +
+                                           std::to_string(getMinFlushTailLength()) + ")");
+        const int64_t b = batch_, t = tailLength;
+        MultiLevelResult r{std::vector<double>((size_t)levels_ * b * t), std::vector<double>((size_t)b * t), levels_, (int)b, (int)t};
+        Engine &e = Engine::get();
+        e.check(vw_stream_flush(e.ctx(), st_, t, r.detailPerLevel.data(), t, b * t, r.finalApprox.data(), t, 0));
+        return r;
+    }
+    int getMinFlushTailLength() const { return (int)hs_.size() - 1; }
+    int getHistoryLengthForLevel(int level) const {
+        if (level < 1 || level > levels_) throw IllegalArgumentException("level must be in [1," + std::to_string(levels_) + "]");
+        return ((int)hs_.size() - 1) << (level - 1);
+    }
+    int suggestFlushTailLength() const { return getMinFlushTailLength(); }
+
+private:
+    BoundaryMode mode_;
+    int levels_;
+    std::vector<double> hs_, gs_;
+    vw_stream_state *st_ = nullptr;
+    int batch_ = 0;
+};
+
 // ---- BatchSIMDMODWT SoA statics (EXT/extensions/modwt/BatchSIMDMODWT.java:64-81,282-308,343-424) -----------------------
 // flat arrays indexed t*batchSize + b; the engine runs on that layout directly (vw_modwt_forward_soa), no transposes
 struct BatchSIMDMODWT {

@@ -101,6 +101,19 @@ public final class VwNative {
     static final MethodHandle vw_modwt_stream_level = h("vw_modwt_stream_level",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, JAVA_LONG, JAVA_LONG, ADDRESS, ADDRESS,
                     JAVA_INT, JAVA_INT, ADDRESS, JAVA_LONG, ADDRESS, JAVA_LONG, JAVA_INT));
+    /** int vw_stream_create(ctx, hs, gs, l, levels, mode, vw_stream_state **out) -- BatchStreamingMODWT's histories in HBM
+     *  (ZERO_PADDING / SYMMETRIC); vw_stream_process runs a block's whole cascade, vw_stream_flush the tail (:55-276) */
+    public static final MethodHandle vw_stream_create = h("vw_stream_create",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS));
+    public static final MethodHandle vw_stream_destroy = h("vw_stream_destroy", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
+    /** int vw_stream_process(ctx, st, x, batch, n, ldx, w, ldw, level_stride_w, v, ldv, flags) */
+    public static final MethodHandle vw_stream_process = h("vw_stream_process",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, JAVA_LONG, ADDRESS, JAVA_LONG,
+                    JAVA_LONG, ADDRESS, JAVA_LONG, JAVA_INT));
+    /** int vw_stream_flush(ctx, st, tail_length, w, ldw, level_stride_w, v, ldv, flags) -- histories not advanced */
+    public static final MethodHandle vw_stream_flush = h("vw_stream_flush",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, JAVA_LONG, JAVA_LONG, ADDRESS, JAVA_LONG, JAVA_INT));
+    public static final MethodHandle vw_stream_reset = h("vw_stream_reset", FunctionDescriptor.of(JAVA_INT, ADDRESS));
 
     // ---- ABI v2: device-resident results, several GPUs from one thread, graph replay (include/vw_modwt.h) -----------
     /** int vw_modwt_decompose_h(ctx, x, batch, n, ldx, hs, gs, l, levels, mode, vw_result **res, flags) */

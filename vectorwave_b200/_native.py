@@ -110,6 +110,11 @@ SIGNATURES = {
     "vw_modwt_forward_soa": (C.c_int, [_vp, _vp, _i64, _i64, _dp, _dp, C.c_int32, C.c_int32, C.POINTER(C.c_void_p), _vp, _u32]),
     "vw_sure_threshold": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _dp, _dp, _u32]),
     "vw_modwt_stream_level": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _dp, _dp, _i32, _i32, _vp, _i64, _vp, _i64, _u32]),
+    "vw_stream_create": (C.c_int, [_vp, _dp, _dp, _i32, _i32, _i32, C.POINTER(_vp)]),
+    "vw_stream_destroy": (C.c_int, [_vp, _vp]),
+    "vw_stream_process": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _u32]),
+    "vw_stream_flush": (C.c_int, [_vp, _vp, _i64, _vp, _i64, _i64, _vp, _i64, _u32]),
+    "vw_stream_reset": (C.c_int, [_vp]),
     "vw_modwt_forward_span": (C.c_int, [_vp, _vp, _i64, _i64, _dp, _dp, _i32, _i32, _i32, _vp, _i64, _vp, _u32]),
     "vw_modwt_inverse_span": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _dp, _dp, _i32, _i32, _i32, _i32, _vp, _u32]),
     "vw_span_halo": (_i64, [_i32, _i32, _i32]),
@@ -652,6 +657,18 @@ class Engine:
                 _vp(v_out.data_ptr()), v_out.stride(0), fl))
         return w_out, v_out
 
+    def stream_create(self, hs, gs, levels, mode):
+        """vw_stream_create: a StreamState keeping every level's history of a blockwise ZERO_PADDING / SYMMETRIC stream
+        in HBM (BatchStreamingMODWT's state)."""
+        hs, gs = _fp(hs), _fp(gs)
+        if hs.size != gs.size:
+            raise IllegalArgumentException("low-pass and high-pass filters must have the same length")
+        st = StreamState(self, int(levels))
+        with self._call_lock:
+            self._check(self.lib.vw_stream_create(self.ctx, hs.ctypes.data_as(_dp), gs.ctypes.data_as(_dp), hs.size,
+                                                  int(levels), int(mode), C.byref(st.handle)))
+        return st
+
     def inverse_span(self, vin_ext, w_ext, halo, hs, gs, first_level, nlevels, order=ORDER_SPLIT, flags=0, out=None):
         """vin_ext [span | halo], w_ext [nlevels][span | halo] (CUDA) -> V_{first-1} [n_local]."""
         import torch
@@ -843,6 +860,64 @@ class DeviceResult:
     def __del__(self):
         try:
             self.free()
+        except Exception:
+            pass
+
+
+class StreamState:
+    """vw_stream_state: the histories of a blockwise stream live in HBM, and every block runs its whole cascade in one
+    call.  Outputs follow the block's residency (numpy / pinned numpy: staged by the engine; CUDA tensor: zero copy)."""
+
+    def __init__(self, eng, levels):
+        self.eng, self.levels, self.handle = eng, levels, _vp()
+        self.batch = None          # rows of the running stream (output shape of flush); None: no block since create / reset
+
+    @staticmethod
+    def _wv(w, v):
+        ldw = w.stride(1) if _is_torch(w) else w.strides[1] // 8
+        lsw = w.stride(0) if _is_torch(w) else w.strides[0] // 8
+        return ldw, lsw, _ld(v)
+
+    def process(self, x, flags=0, w_out=None, v_out=None):
+        """block [B][n] -> (W [levels][B][n], V_J [B][n]); advances every level's history."""
+        x2, _ = Engine._rows(x, "block")
+        b, n = x2.shape
+        w = w_out if w_out is not None else Engine._empty_like_rows(x2, self.levels, b, max(n, 1))
+        v = v_out if v_out is not None else Engine._empty_like_rows(x2, b, max(n, 1))
+        ldw, lsw, ldv = self._wv(w, v)
+        with self.eng._call_lock:
+            fl = self.eng._bind_stream(x2, w, v) | flags
+            self.eng._check(self.eng.lib.vw_stream_process(self.eng.ctx, self.handle, _vp(_ptr(x2)), b, n, _ld(x2), _vp(_ptr(w)),
+                                                           ldw, lsw, _vp(_ptr(v)), ldv, fl))
+        self.batch = b
+        return w, v
+
+    def flush(self, tail_length, flags=0, w_out=None, v_out=None):
+        """the cascade over the flush tail (histories not advanced) -> (W [levels][batch][tail], V_J [batch][tail]);
+        host arrays unless CUDA tensors are given as outputs"""
+        t, batch = max(int(tail_length), 1), self.batch or 1
+        w = w_out if w_out is not None else np.empty((self.levels, batch, t))
+        v = v_out if v_out is not None else np.empty((batch, t))
+        ldw, lsw, ldv = self._wv(w, v)
+        with self.eng._call_lock:
+            fl = self.eng._bind_stream(w, v) | flags
+            self.eng._check(self.eng.lib.vw_stream_flush(self.eng.ctx, self.handle, int(tail_length), _vp(_ptr(w)), ldw, lsw,
+                                                         _vp(_ptr(v)), ldv, fl))
+        return w, v
+
+    def reset(self):
+        self.eng._check(self.eng.lib.vw_stream_reset(self.handle))
+        self.batch = None
+
+    def close(self):
+        if self.handle:
+            with self.eng._call_lock:
+                self.eng.lib.vw_stream_destroy(self.eng.ctx, self.handle)
+            self.handle = _vp()
+
+    def __del__(self):
+        try:
+            self.close()
         except Exception:
             pass
 

@@ -159,6 +159,8 @@ int inverse_device(vw_ctx *ctx, const double *w, int64_t ldw, int64_t lsw, const
                    int64_t n, const VwFilt &f, int l, int levels, int mode, const vw_align *align, int order,
                    uint64_t detail_mask, int use_approx, double *xout, int64_t ldx, uint32_t flags, const double *thr_dev,
                    int thr_per_row, int thr_soft, int64_t thr_lstride);
+int stream_level_device(vw_ctx *ctx, const double *vin, int64_t batch, int64_t ldin, int64_t hist, int64_t n, const VwFilt &f,
+                        int l, int level, double *w, int64_t ldw, double *v, int64_t ldv, uint32_t flags);
 }  // namespace vwshim
 int vw_cuda_check(vw_ctx *ctx, cudaError_t e, const char *what);
 int vw_scratch(vw_ctx *ctx, int slot, size_t bytes, void **out);

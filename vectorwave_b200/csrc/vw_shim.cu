@@ -204,6 +204,29 @@ int finish(vw_ctx *ctx, uint32_t flags, bool host_io) {
 
 vw_align default_align() { return vw_align{1, 0, 1, 0}; }
 
+// One level of a streaming block over [history | block] rows (vw_modwt_stream_level and the per-level path of the
+// stream state): the row is a linear span, so the tile kernel (any dilation whose halo fits) or, for deep levels, the
+// column kernel -- the same kernels as the whole-signal path -- and the generic kernel for the rest and for BITEXACT.
+int stream_level_device(vw_ctx *ctx, const double *vin, int64_t batch, int64_t ldin, int64_t hist, int64_t n, const VwFilt &f,
+                        int l, int level, double *w, int64_t ldw, double *v, int64_t ldv, uint32_t flags) {
+    const int64_t d = (int64_t)1 << (level - 1), n_in = hist + n;
+    const bool exact = flags & VW_FLAG_BITEXACT;
+    ctx->plan_lean_ok = true;
+    int rc = VW_EUNSUPPORTED;
+    if (!exact && !(flags & VW_FLAG_NO_FUSE)) {
+        VwFusedFwd p{vin, ldin, w, ldw, 0, v, ldv, batch, n_in, hist, n, l, level, 1, VW_MODE_LINEAR, 0};
+        rc = vw_fused_forward(ctx, p, f);
+        if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
+        if (rc == VW_EUNSUPPORTED && d >= 4 && ctx->opt_poly != 0) {
+            rc = vw_column_analysis(ctx, vin, ldin, v, ldv, w, ldw, n_in, hist, n, batch, f, l, d, VW_MODE_LINEAR);
+            if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
+        }
+    }
+    if (rc == VW_EUNSUPPORTED)
+        rc = vw_launch_analysis_level(ctx, vin, ldin, v, ldv, w, ldw, n_in, hist, n, batch, f, l, d, VW_MODE_LINEAR, exact);
+    return rc;
+}
+
 // Analysis cascade over device buffers.  Groups of levels come from the planner; a group the fused kernel declines
 // (unaligned rows, exotic filter length, ...) runs level by level on the generic kernels.
 int forward_device(vw_ctx *ctx, const double *x, int64_t batch, int64_t n, int64_t ldx, const VwFilt &f, int l,
@@ -1510,24 +1533,8 @@ int vw_modwt_stream_level(vw_ctx *ctx, const double *vin, int64_t batch, int64_t
     const int64_t need = (int64_t)(l - 1) * d;
     if (hist < need) return vw_fail(ctx, VW_ELENGTH, "history %lld shorter than the %lld samples level %d needs",
                                     (long long)hist, (long long)need, level);
-    const int64_t n_in = hist + n;
-    if (ldin < n_in || ldw < n || ldv < n) return vw_fail(ctx, VW_ELENGTH, "row stride shorter than the row");
-    const bool exact = flags & VW_FLAG_BITEXACT;
-    rc = VW_EUNSUPPORTED;
-    if (!exact && !(flags & VW_FLAG_NO_FUSE)) {
-        // the [history | block] row is a linear span: the tile kernel (any dilation whose halo fits) or, for deep
-        // levels, the column kernel -- the same kernels as the whole-signal path
-        VwFusedFwd p{vin, ldin, w, ldw, 0, v, ldv, batch, n_in, hist, n, l, level, 1, VW_MODE_LINEAR, 0};
-        rc = vw_fused_forward(ctx, p, f);
-        if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
-        if (rc == VW_EUNSUPPORTED && d >= 4 && ctx->opt_poly != 0) {
-            rc = vw_column_analysis(ctx, vin, ldin, v, ldv, w, ldw, n_in, hist, n, batch, f, l, d, VW_MODE_LINEAR);
-            if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
-        }
-    }
-    if (rc == VW_EUNSUPPORTED)
-        rc = vw_launch_analysis_level(ctx, vin, ldin, v, ldv, w, ldw, n_in, hist, n, batch, f, l, d, VW_MODE_LINEAR, exact);
-    if (rc) return rc;
+    if (ldin < hist + n || ldw < n || ldv < n) return vw_fail(ctx, VW_ELENGTH, "row stride shorter than the row");
+    if ((rc = stream_level_device(ctx, vin, batch, ldin, hist, n, f, l, level, w, ldw, v, ldv, flags))) return rc;
     return finish(ctx, flags, false);
 }
 

@@ -1,28 +1,21 @@
 """BatchStreamingMODWT over the native engine (EXT/extensions/modwt/BatchStreamingMODWT.java).
 
-Blockwise batch MODWT with a carried left history per level: every level keeps the last
-(L-1)*2^(j-1) samples of ITS input on the device, so consecutive blocks continue each other exactly
-(ZERO_PADDING: zeros before the stream; SYMMETRIC: the first block reflected about its left edge, per level,
-:326-334).  PERIODIC has no state: each block is transformed on its own, like the reference (:62-64,113-115).
+Blockwise batch MODWT with a carried left history per level: every level keeps the last (L-1)*2^(j-1) samples of ITS
+input, so consecutive blocks continue each other exactly (ZERO_PADDING: zeros before the stream; SYMMETRIC: the first
+block reflected about its left edge, per level, :326-334).  PERIODIC has no state: each block is transformed on its own,
+like the reference (:62-64,113-115).
 
-Layout on the device: level j owns one buffer ext_j [B][hist_j + n] of [history | block] rows.  The block part of
-ext_{j+1} IS the approximation output of level j (vw_modwt_stream_level writes V there), so the cascade makes no
-copies; after a block the tail of every ext_j slides into its history part.
+The histories live in HBM behind one native stream state (vw_stream_state): a block's whole cascade, the first-block
+initialisation, the batch-size restart and the flush tail all run below the C ABI, so this class only validates,
+chooses the residency of the results and raises the reference's exceptions.
 """
 import numpy as np
 
-from . import _native
 from ._native import Engine
 from .batch import BatchMODWT, MultiLevelResult, SingleLevelResult, _validate_aos
 from .errors import IllegalArgumentException
 from .modwt import SCALE, _is_torch
 from .wavelets import BoundaryMode
-
-
-def _mirror(idx, n):
-    """MathUtils.symmetricBoundaryExtension (CORE/util/MathUtils.java:30-51)"""
-    m = np.mod(idx, 2 * n)
-    return np.where(m < n, m, 2 * n - 1 - m)
 
 
 class UnsupportedOperationException(RuntimeError):
@@ -68,67 +61,25 @@ class BatchStreamingMODWT:
         self._gs = self.wavelet.highPassDecomposition() * SCALE
         l = self._hs.size
         self._hist_len = [(l - 1) * (1 << j) for j in range(self.levels)]   # filterLen(level) - 1, :302-303
-        self._hist = None         # per level: torch [B][hist_j] (device), None until initialised
-        self._last_batch = -1
+        self._state = None        # native stream state, created by the first block
 
     # ---- helpers ------------------------------------------------------------------------------------------
     def _eng(self):
         return self._engine or Engine.get()
 
-    def _to_device(self, block):
-        import torch
-        if _is_torch(block):
-            return block.to(dtype=torch.float64, device=f"cuda:{self._eng().device}").contiguous(), True
-        return torch.as_tensor(np.ascontiguousarray(block), device=f"cuda:{self._eng().device}"), False
-
-    @staticmethod
-    def _to_caller(t, was_torch):
-        return t if was_torch else t.cpu().numpy()
-
     def _ensure_levels(self, expected):
         if self.levels != expected:
             raise IllegalStateException(f"This instance is configured for levels={self.levels}, expected={expected}")
 
-    def _ensure_history_capacity(self, batch):
-        """:306-320 -- a batch-size change restarts the stream (histories are re-initialised from the next block)."""
-        if self._hist is None:
-            self._hist = [None] * self.levels
-        elif self._last_batch != batch:
-            self._hist = [None] * self.levels
-        self._last_batch = batch
-
-    def _init_history(self, level_index, cur):
-        """first block of a stream at this level: zeros, or the level input reflected about its left edge (:326-334)"""
-        import torch
-        b, n = cur.shape
-        hl = self._hist_len[level_index]
-        if self.boundaryMode == BoundaryMode.ZERO_PADDING:
-            return torch.zeros((b, hl), dtype=torch.float64, device=cur.device)
-        src = _mirror(np.arange(hl) - hl, n)
-        return cur[:, torch.as_tensor(src, device=cur.device)].contiguous()
-
-    def _cascade(self, x, nlevels):
-        """x: device [B][n].  Returns (W [nlevels][B][n], V [B][n]) and advances every level's history."""
-        import torch
+    def _process(self, x):
+        """x: validated [B][n] block (numpy or torch) -> (W [levels][B][n], V [B][n]) in the block's residency"""
         eng = self._eng()
-        b, n = x.shape
-        w = torch.empty((nlevels, b, n), dtype=torch.float64, device=x.device)
-        v_final = torch.empty((b, n), dtype=torch.float64, device=x.device)
-        exts = [torch.empty((b, self._hist_len[j] + n + (self._hist_len[j] + n) % 2), dtype=torch.float64, device=x.device)
-                for j in range(nlevels)]   # even row stride keeps the rows 16-byte aligned for the bulk copies
-        exts[0][:, self._hist_len[0]:self._hist_len[0] + n] = x
-        for j in range(nlevels):
-            hl = self._hist_len[j]
-            ext = exts[j][:, :hl + n]
-            block = ext[:, hl:]
-            if self._hist[j] is None:
-                self._hist[j] = self._init_history(j, block)
-            ext[:, :hl] = self._hist[j]
-            v_out = exts[j + 1][:, self._hist_len[j + 1]:self._hist_len[j + 1] + n] if j + 1 < nlevels else v_final
-            eng.stream_level(ext, hl, self._hs, self._gs, j + 1, w[j], v_out)
-            # updateHistoryFromSoA (:336-350): the last hl samples of [history | block]
-            self._hist[j] = ext[:, n:n + hl].clone()
-        return w, v_final
+        if _is_torch(x):
+            import torch
+            x = x.to(dtype=torch.float64, device=f"cuda:{eng.device}").contiguous()
+        if self._state is None:
+            self._state = eng.stream_create(self._hs, self._gs, self.levels, self.boundaryMode.value)
+        return self._state.process(x)
 
     # ---- API ----------------------------------------------------------------------------------------------
     def processSingleLevel(self, block):
@@ -137,68 +88,48 @@ class BatchStreamingMODWT:
         x = _validate_aos(block)
         if self.boundaryMode == BoundaryMode.PERIODIC:
             return BatchMODWT.singleLevelAoS(self.wavelet, x, self._engine)
-        xd, was_torch = self._to_device(x)
-        self._ensure_history_capacity(xd.shape[0])
-        w, v = self._cascade(xd, 1)
-        return SingleLevelResult(self._to_caller(v, was_torch), self._to_caller(w[0], was_torch))
+        w, v = self._process(x)
+        return SingleLevelResult(v, w[0])
 
     def processMultiLevel(self, block):
         """:111-163"""
         x = _validate_aos(block)
         if self.boundaryMode == BoundaryMode.PERIODIC:
             return BatchMODWT.multiLevelAoS(self.wavelet, x, self.levels, self._engine)
-        xd, was_torch = self._to_device(x)
-        self._ensure_history_capacity(xd.shape[0])
-        w, v = self._cascade(xd, self.levels)
-        return MultiLevelResult(self._to_caller(w, was_torch), self._to_caller(v, was_torch))
+        w, v = self._process(x)
+        return MultiLevelResult(w, v)
 
-    def _tail(self, tail_length):
-        """buildTailFromHistorySoA (:358-372): zeros, or the last samples reflected about the end of the stream"""
-        import torch
-        h0 = self._hist[0]
-        if self.boundaryMode == BoundaryMode.ZERO_PADDING:
-            return torch.zeros((h0.shape[0], tail_length), dtype=torch.float64, device=h0.device)
-        idx = torch.arange(h0.shape[1] - 1, h0.shape[1] - 1 - tail_length, -1, device=h0.device)
-        return h0[:, idx].contiguous()
-
-    def _flush(self, tail_length, nlevels):
+    def _flush(self, tail_length):
+        """the cascade over buildTailFromHistorySoA's tail (:358-372); the histories are not advanced (:205-222,252-274)"""
         if self.boundaryMode == BoundaryMode.PERIODIC:
             raise UnsupportedOperationException("Flush is only applicable to ZERO_PADDING/SYMMETRIC")
         if tail_length <= 0:
             return None
-        if self._hist is None:
+        if self._state is None or self._state.batch is None:
             raise IllegalStateException("No prior blocks processed; cannot flush")
-        for j in range(nlevels):
-            if self._hist[j] is None:
-                raise IllegalStateException(f"History not initialized at level {j + 1}")
-        limit = min(self._hist_len[:nlevels])
+        limit = min(self._hist_len)
         if tail_length > limit:
             raise IllegalArgumentException(
                 f"tailLength ({tail_length}) exceeds maximum allowed across levels ({limit}). "
                 "Use getMinFlushTailLength() to choose a valid tail length.")
-        # the reference's flush does not advance the histories (:205-222,252-274): work on copies
-        saved = [h.clone() for h in self._hist]
-        try:
-            return self._cascade(self._tail(tail_length), nlevels)
-        finally:
-            self._hist = saved
+        return self._state.flush(tail_length)
 
     def flushSingleLevel(self, tailLength):
         """:183-222"""
         self._ensure_levels(1)
-        r = self._flush(tailLength, 1)
+        r = self._flush(tailLength)
         if r is None:
             return SingleLevelResult(np.zeros((0, 0)), np.zeros((0, 0)))
         w, v = r
-        return SingleLevelResult(v.cpu().numpy(), w[0].cpu().numpy())
+        return SingleLevelResult(v, w[0])
 
     def flushMultiLevel(self, tailLength):
         """:231-276"""
-        r = self._flush(tailLength, self.levels)
+        r = self._flush(tailLength)
         if r is None:
             return MultiLevelResult(np.zeros((self.levels, 0, 0)), np.zeros((0, 0)))
         w, v = r
-        return MultiLevelResult(w.cpu().numpy(), v.cpu().numpy())
+        return MultiLevelResult(w, v)
 
     def getMinFlushTailLength(self):
         return min(self._hist_len)
@@ -212,7 +143,9 @@ class BatchStreamingMODWT:
         return self._hist_len[0] if self.levels == 1 else min(self._hist_len)
 
     def close(self):
-        self._hist = None
+        if self._state is not None:
+            self._state.close()
+            self._state = None
 
     def __enter__(self):
         return self
