@@ -377,6 +377,33 @@ VW_API int vw_span_unpack_inverse(vw_ctx *ctx, const vw_span_plan *plan, const d
 VW_API int vw_modwt_inverse_span_all(vw_ctx *ctx, const vw_span_plan *plan, const double *w, int64_t row_stride,
                               const double *v, const double *hs, const double *gs, int32_t order, double *xout,
                               uint32_t flags);
+/* The same synthesis of the soft (soft != 0) or hard thresholded W: thr_dev is ONE device double, applied to every W
+ * sample the kernels load -- the halo included, which holds the neighbour's raw coefficients that the neighbour thresholds
+ * on load too, so the ranks together give the whole-signal synthesis of the thresholded coefficients.  V_J is not
+ * thresholded; W and V are read only (the per-level kernels of VW_FLAG_BITEXACT / VW_FLAG_NO_FUSE threshold a scratch copy). */
+VW_API int vw_modwt_inverse_span_all_thr(vw_ctx *ctx, const vw_span_plan *plan, const double *w, int64_t row_stride,
+                                         const double *v, const double *hs, const double *gs, int32_t order,
+                                         const double *thr_dev, int32_t soft, double *xout, uint32_t flags);
+
+/* ---- exact median of |c| over a signal split into spans (the universal threshold of a span-sharded signal) ---------- */
+/* The seven digit rounds of vw_universal_threshold's selection with the histogram reduction left to the caller, so ranks
+ * in separate processes (NCCL, one GPU each) can drive it.  Per rank: allocate vw_span_median_state_bytes(n_local) bytes of
+ * device memory, vw_span_median_init once, then for round = 0 .. VW_SPAN_MEDIAN_ROUNDS-1:
+ *   vw_span_median_hist(own span -> hist, vw_span_median_bins(round) uint64 entries);
+ *   the caller sums hist over the ranks (e.g. ncclAllReduce with ncclUint64 / ncclSum) into hist_sum;
+ *   vw_span_median_pick(hist_sum)  -- every rank picks from the identical sum, so every rank's state stays identical;
+ * finally vw_span_median_value writes median(|c|) / 0.6745 * factor, or the raw median for factor < 0 (even n_total: the mean
+ * of the two middle order statistics), to one device double.  The universal threshold uses factor = sqrt(2 ln n_total).
+ * Candidate buffers stay rank-local: a rank whose round-2 bucket overflows them (a constant span) histograms its full span
+ * in the later rounds, the sum is still exact.  All pointers are device pointers on ctx's device; every call only
+ * enqueues on ctx's stream and nothing synchronises. */
+#define VW_SPAN_MEDIAN_ROUNDS 7
+VW_API int32_t vw_span_median_bins(int32_t round);   /* 2 * 4096 (rounds 0, 1), 2 * 256 (rounds 2..6), 0 outside */
+VW_API size_t vw_span_median_state_bytes(int64_t n_local);
+VW_API int vw_span_median_init(vw_ctx *ctx, void *state, int64_t n_total);
+VW_API int vw_span_median_hist(vw_ctx *ctx, void *state, const double *c, int64_t n_local, int32_t round, uint64_t *hist);
+VW_API int vw_span_median_pick(vw_ctx *ctx, void *state, int32_t round, const uint64_t *hist_sum);
+VW_API int vw_span_median_value(vw_ctx *ctx, const void *state, double factor, double *out_dev);
 
 /* ---- several GPUs driven by ONE host thread (the JVM case) ------------------------------------------------------ */
 /* vw_init_multi opens one ctx per listed device and enables peer access between ring neighbours.  The sharded calls
@@ -401,6 +428,20 @@ VW_API int vw_modwt_forward_sharded(vw_multi *m, const vw_span_plan *plan, doubl
 VW_API int vw_modwt_inverse_sharded(vw_multi *m, const vw_span_plan *plan, double *const *w, int64_t row_stride,
                              double *const *v, const double *hs, const double *gs, int32_t mode, int32_t order,
                              double *const *xout, float *exchange_ms, uint32_t flags);
+/* VectorWaveSwtAdapter.denoise (CORE/swt/VectorWaveSwtAdapter.java:532-562) of ONE signal of world * n_local samples spread
+ * over the devices, i.e. vw_swt_denoise with batch = 1 on the whole signal: vw_modwt_forward_sharded, then (threshold < 0)
+ * the universal threshold median(|W_1|)/0.6745 * sqrt(2 ln N) with the exact median over all ranks (the vw_span_median_*
+ * rounds, histograms summed on the devices: every device pulls the others' tables with cudaMemcpyPeerAsync, ordered by
+ * events, no host round trip between rounds) or the fixed `threshold`, then the synthesis exchange and
+ * vw_modwt_inverse_span_all_thr on every device.  The same threshold applies to every detail level; V_J is untouched.
+ * Buffers as vw_modwt_forward_sharded / vw_modwt_inverse_sharded (w and v receive the raw coefficients).
+ * VW_FLAG_CHECK_FINITE checks every span first: VW_ENONFINITE names the rank and nothing is written to xout.
+ * threshold_out (may be NULL): the threshold on the HOST (for the universal threshold this waits for rank 0's stream).
+ * One synchronise at the end, none with VW_FLAG_NO_SYNC (vw_multi_synchronize then waits). */
+VW_API int vw_swt_denoise_sharded(vw_multi *m, const vw_span_plan *plan, double *const *xext, const double *hs,
+                                  const double *gs, int32_t mode, int32_t order, double threshold, int32_t soft,
+                                  double *const *w, int64_t row_stride, double *const *v, double *const *xout,
+                                  double *threshold_out, uint32_t flags);
 
 /* ---- device-resident results (MultiLevelMODWTResult kept on the GPU between calls) ------------------------------ */
 /* CORE/modwt/MultiLevelMODWTResultImpl.java:51-139 and MutableMultiLevelMODWTResultImpl are opaque enough to be backed

@@ -461,6 +461,26 @@ public:
         for (size_t r = 0; r < world; r++) chk(r, vw_copy_d2h(vw_multi_ctx(m_, (int)r), x.data() + r * n_, out_[r], (size_t)n_ * 8));
         return x;
     }
+    // VectorWaveSwtAdapter.denoise of the whole signal (vw_swt_denoise_sharded): threshold < 0 selects the universal
+    // threshold from the exact median of |W_1| over every span; *threshold_out (may be null) receives the value used.
+    // The coefficients stay on the devices unthresholded, so reconstruct() afterwards gives the plain reconstruction.
+    std::vector<double> denoise(const std::vector<double> &signal, double threshold = -1.0, bool soft = true,
+                                double *threshold_out = nullptr) {
+        const size_t world = xext_.size(), total = world * (size_t)n_;
+        if (signal.size() != total) throw IllegalArgumentException("signal length must be world * n_local");
+        for (size_t r = 0; r < world; r++)
+            chk(r, vw_copy_h2d(vw_multi_ctx(m_, (int)r), xext_[r] + plan_.lead, signal.data() + r * n_, (size_t)n_ * 8));
+        double thr = 0.0;
+        const int rc = vw_swt_denoise_sharded(m_, &plan_, xext_.data(), hs_.data(), gs_.data(), (int)mode_,
+                                              mode_ == BoundaryMode::ZERO_PADDING ? VW_ORDER_PAIR : VW_ORDER_SPLIT, threshold,
+                                              soft ? 1 : 0, w_.data(), row_, v_.data(), out_.data(), &thr, VW_FLAG_CHECK_FINITE);
+        if (rc == VW_ENONFINITE) throw InvalidSignalException(vw_multi_last_error(m_), "VAL_003");
+        mchk(rc);
+        if (threshold_out) *threshold_out = thr;
+        std::vector<double> x(total);
+        for (size_t r = 0; r < world; r++) chk(r, vw_copy_d2h(vw_multi_ctx(m_, (int)r), x.data() + r * n_, out_[r], (size_t)n_ * 8));
+        return x;
+    }
 
 private:
     void mchk(int rc) const { if (rc != VW_OK) throw NativeEngineError(vw_multi_last_error(m_)); }

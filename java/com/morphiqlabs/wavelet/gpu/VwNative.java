@@ -157,6 +157,28 @@ public final class VwNative {
     public static final MethodHandle vw_modwt_inverse_sharded = h("vw_modwt_inverse_sharded",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, ADDRESS,
                     ADDRESS, JAVA_INT));
+    /** int vw_swt_denoise_sharded(m, plan, xext, hs, gs, mode, order, threshold, soft, w, row_stride, v, xout,
+     *  double *threshold_out, flags): one long signal denoised across the devices with the exact universal threshold */
+    public static final MethodHandle vw_swt_denoise_sharded = h("vw_swt_denoise_sharded",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_DOUBLE, JAVA_INT,
+                    ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS, JAVA_INT));
+    /** int vw_modwt_inverse_span_all_thr(ctx, plan, w, row_stride, v, hs, gs, order, const double *thr_dev, soft, xout, flags) */
+    public static final MethodHandle vw_modwt_inverse_span_all_thr = h("vw_modwt_inverse_span_all_thr",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, JAVA_INT,
+                    ADDRESS, JAVA_INT));
+    /** The cross-rank median rounds (one process per GPU): state_bytes(n_local); init(ctx, state, n_total); for round in
+     *  0 .. SPAN_MEDIAN_ROUNDS-1: hist(ctx, state, c, n_local, round, uint64 *hist) -> caller's all-reduce (sum) ->
+     *  pick(ctx, state, round, const uint64 *hist_sum); value(ctx, state, factor, double *out_dev).  Device pointers. */
+    public static final int SPAN_MEDIAN_ROUNDS = 7;
+    public static final MethodHandle vw_span_median_bins = h("vw_span_median_bins", FunctionDescriptor.of(JAVA_INT, JAVA_INT));
+    public static final MethodHandle vw_span_median_state_bytes = h("vw_span_median_state_bytes", FunctionDescriptor.of(JAVA_LONG, JAVA_LONG));
+    public static final MethodHandle vw_span_median_init = h("vw_span_median_init", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG));
+    public static final MethodHandle vw_span_median_hist = h("vw_span_median_hist",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, ADDRESS));
+    public static final MethodHandle vw_span_median_pick = h("vw_span_median_pick",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS));
+    public static final MethodHandle vw_span_median_value = h("vw_span_median_value",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_DOUBLE, ADDRESS));
     /** CUDA-graph replay of a fixed call sequence: vw_graph_begin(ctx); ...calls...; vw_graph_end(ctx, &g); vw_graph_launch(ctx, g, flags) */
     public static final MethodHandle vw_graph_begin = h("vw_graph_begin", FunctionDescriptor.of(JAVA_INT, ADDRESS));
     public static final MethodHandle vw_graph_end = h("vw_graph_end", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));

@@ -123,6 +123,14 @@ SIGNATURES = {
     "vw_span_pack_inverse": (C.c_int, [_vp, C.POINTER(VwSpanPlan), _vp, _i64, _vp, _vp, _u32]),
     "vw_span_unpack_inverse": (C.c_int, [_vp, C.POINTER(VwSpanPlan), _vp, _vp, _i64, _vp, _u32]),
     "vw_modwt_inverse_span_all": (C.c_int, [_vp, C.POINTER(VwSpanPlan), _vp, _i64, _vp, _dp, _dp, _i32, _vp, _u32]),
+    "vw_modwt_inverse_span_all_thr": (C.c_int, [_vp, C.POINTER(VwSpanPlan), _vp, _i64, _vp, _dp, _dp, _i32, _vp, _i32, _vp,
+                                                _u32]),
+    "vw_span_median_bins": (_i32, [_i32]),
+    "vw_span_median_state_bytes": (C.c_size_t, [_i64]),
+    "vw_span_median_init": (C.c_int, [_vp, _vp, _i64]),
+    "vw_span_median_hist": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _vp]),
+    "vw_span_median_pick": (C.c_int, [_vp, _vp, _i32, _vp]),
+    "vw_span_median_value": (C.c_int, [_vp, _vp, C.c_double, _vp]),
     "vw_init_multi": (C.c_int, [C.POINTER(C.c_int), _i32, C.POINTER(_vp)]),
     "vw_destroy_multi": (C.c_int, [_vp]),
     "vw_multi_size": (_i32, [_vp]),
@@ -133,6 +141,8 @@ SIGNATURES = {
                                            C.POINTER(_vp), C.POINTER(C.c_float), _u32]),
     "vw_modwt_inverse_sharded": (C.c_int, [_vp, C.POINTER(VwSpanPlan), C.POINTER(_vp), _i64, C.POINTER(_vp), _dp, _dp, _i32,
                                            _i32, C.POINTER(_vp), C.POINTER(C.c_float), _u32]),
+    "vw_swt_denoise_sharded": (C.c_int, [_vp, C.POINTER(VwSpanPlan), C.POINTER(_vp), _dp, _dp, _i32, _i32, C.c_double, _i32,
+                                         C.POINTER(_vp), _i64, C.POINTER(_vp), C.POINTER(_vp), _dp, _u32]),
     "vw_modwt_decompose_h": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _dp, _dp, _i32, _i32, _i32, C.POINTER(_vp), _u32]),
     "vw_result_shape": (C.c_int, [_vp, C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_i32)]),
     "vw_result_get_level": (C.c_int, [_vp, _vp, _i32, _vp, _i64, _u32]),
@@ -716,6 +726,52 @@ class Engine:
                                                            _vp(v.data_ptr()), hs.ctypes.data_as(_dp), gs.ctypes.data_as(_dp),
                                                            int(order), _vp(out.data_ptr()), fl))
 
+    def inverse_span_all_thr(self, plan, w, v, hs, gs, order, thr, soft, out, flags=0):
+        """inverse_span_all of the thresholded W: thr is a one-element float64 CUDA tensor (the threshold stays on the
+        device), applied to every W sample as the kernels load it; W and V are left as they are."""
+        hs, gs = _fp(hs), _fp(gs)
+        with self._call_lock:
+            fl = self._bind_stream(w, v, thr, out) | flags
+            self._check(self.lib.vw_modwt_inverse_span_all_thr(self.ctx, C.byref(plan), _vp(w.data_ptr()), w.stride(0),
+                                                               _vp(v.data_ptr()), hs.ctypes.data_as(_dp), gs.ctypes.data_as(_dp),
+                                                               int(order), _vp(thr.data_ptr()), int(bool(soft)),
+                                                               _vp(out.data_ptr()), fl))
+
+    # -- exact median of |c| over spans on several ranks (vw_span_median_*; device tensors, nothing synchronises) -----
+    def span_median_state(self, n_local):
+        """a device state blob for the median rounds of a span of n_local samples (uint8 CUDA tensor)"""
+        import torch
+        return torch.empty(int(self.lib.vw_span_median_state_bytes(int(n_local))), dtype=torch.uint8,
+                           device=torch.device("cuda", self.device))
+
+    def span_median_init(self, state, n_total):
+        with self._call_lock:
+            self._bind_torch_stream()
+            self._check(self.lib.vw_span_median_init(self.ctx, _vp(state.data_ptr()), int(n_total)))
+
+    def span_median_hist(self, state, c, rnd, hist):
+        """histogram of this rank's span c (float64 CUDA, contiguous) for round `rnd` into hist (int64 CUDA tensor of
+        span_median_bins(rnd) entries; the counts are unsigned 64-bit, far below 2^63)"""
+        with self._call_lock:
+            self._bind_torch_stream()
+            self._check(self.lib.vw_span_median_hist(self.ctx, _vp(state.data_ptr()), _vp(c.data_ptr()), int(c.numel()), int(rnd),
+                                                     _vp(hist.data_ptr())))
+
+    def span_median_pick(self, state, rnd, hist_sum):
+        with self._call_lock:
+            self._bind_torch_stream()
+            self._check(self.lib.vw_span_median_pick(self.ctx, _vp(state.data_ptr()), int(rnd), _vp(hist_sum.data_ptr())))
+
+    def span_median_value(self, state, factor, out):
+        """out (one float64 CUDA element) = median / 0.6745 * factor, or the raw median for factor < 0"""
+        with self._call_lock:
+            self._bind_torch_stream()
+            self._check(self.lib.vw_span_median_value(self.ctx, _vp(state.data_ptr()), float(factor), _vp(out.data_ptr())))
+
+    def _bind_torch_stream(self):
+        import torch
+        self._check(self.lib.vw_set_stream(self.ctx, _vp(torch.cuda.current_stream(self.device).cuda_stream)))
+
     # -- timing record / graph replay ----------------------------------------------------------------------
     def last_timing(self):
         """(device_ms, host_ms, launches) of the last public call; needs set_option("timing", 1)."""
@@ -748,6 +804,14 @@ class Engine:
                                                       gs.ctypes.data_as(_dp), hs.size, int(levels), int(mode),
                                                       C.byref(res.handle), fl))
         return res
+
+
+SPAN_MEDIAN_ROUNDS = 7      # VW_SPAN_MEDIAN_ROUNDS
+
+
+def span_median_bins(rnd):
+    """entries of round rnd's histogram (two tables: the lower and the upper middle order statistic)"""
+    return int(load_library().vw_span_median_bins(int(rnd)))
 
 
 def span_plan(l, levels, n_local, world):
@@ -960,6 +1024,18 @@ class MultiEngine:
                                                       hs.ctypes.data_as(_dp), gs.ctypes.data_as(_dp), int(mode), int(order),
                                                       self._ptrs(xout), C.byref(ms) if timed else None, flags))
         return float(ms.value) if timed else None
+
+    def denoise(self, plan, xext, hs, gs, mode, order, w, v, xout, threshold=-1.0, soft=True, flags=0):
+        """vw_swt_denoise_sharded: buffers as forward / inverse (xext filled behind the lead); returns the threshold, or
+        None under FLAG_NO_SYNC (reading it back would wait for rank 0)"""
+        hs, gs = _fp(hs), _fp(gs)
+        thr = C.c_double(0.0)
+        want = not (flags & FLAG_NO_SYNC)
+        self._check(self.lib.vw_swt_denoise_sharded(self.handle, C.byref(plan), self._ptrs(xext), hs.ctypes.data_as(_dp),
+                                                    gs.ctypes.data_as(_dp), int(mode), int(order), float(threshold), int(bool(soft)),
+                                                    self._ptrs(w), w[0].stride(0), self._ptrs(v), self._ptrs(xout),
+                                                    C.byref(thr) if want else None, flags))
+        return float(thr.value) if want else None
 
     def synchronize(self):
         self._check(self.lib.vw_multi_synchronize(self.handle))

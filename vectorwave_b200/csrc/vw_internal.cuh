@@ -99,7 +99,7 @@ struct vw_ctx {
     std::vector<OccEntry> occ_cache;   // occupancy queries of the tile kernels (vw_fused.cu: prefetch_distance)
     int64_t opt_lean = 3;    // issue-lean tile kernels (vw_lean.cu): bit 0 = filters up to 12 taps, bit 1 = 16..20-tap quadrature-mirror pairs
     // set by the cascade drivers for the duration of a call: can this call's tile launches take the lean kernels at all
-    // (not SYMMETRIC, no threshold-on-load, full detail mask)?  The planner budgets shared memory / registers / threads for
+    // (not SYMMETRIC, full detail mask; threshold-on-load is fine: the lean synthesis thresholds every W tile as it lands)?  The planner budgets shared memory / registers / threads for
     // the kernels that will really run.
     bool plan_lean_ok = true;
     int64_t opt_lean_small = 1;   // lean short filters: 128-thread CTAs on ~1024-sample tiles (vw_fused.cu: lean_small_tiles)
@@ -161,6 +161,9 @@ int inverse_device(vw_ctx *ctx, const double *w, int64_t ldw, int64_t lsw, const
                    int thr_per_row, int thr_soft, int64_t thr_lstride);
 int stream_level_device(vw_ctx *ctx, const double *vin, int64_t batch, int64_t ldin, int64_t hist, int64_t n, const VwFilt &f,
                         int l, int level, double *w, int64_t ldw, double *v, int64_t ldv, uint32_t flags);
+int inverse_span_device(vw_ctx *ctx, const double *vin, const double *w, int64_t level_stride_w, int64_t halo, int64_t n_local,
+                        const double *hs, const double *gs, int32_t l, int32_t first_level, int32_t nlevels, int32_t order,
+                        double *vout, uint32_t flags, const double *thr_dev, int32_t thr_soft);
 }  // namespace vwshim
 int vw_cuda_check(vw_ctx *ctx, cudaError_t e, const char *what);
 int vw_scratch(vw_ctx *ctx, int slot, size_t bytes, void **out);
@@ -254,6 +257,11 @@ int vw_launch_universal_threshold(vw_ctx *ctx, const double *w1, int64_t batch, 
                                   double *thr_dev);
 // same selection, raw median(|c|) per row
 int vw_launch_median_abs(vw_ctx *ctx, const double *c, int64_t batch, int64_t n, int64_t ld, double *med_dev);
+// the span median's cross-rank reduction on the device (vw_swt_denoise_sharded): out = own + the other ranks' tables of
+// gather[ranks][entries] (slot `self` is not read), and a fixed threshold stored without a host copy
+int vw_launch_span_hist_sum(vw_ctx *ctx, const uint64_t *gather, const uint64_t *own, int ranks, int self, int entries,
+                            uint64_t *out);
+int vw_launch_span_fixed(vw_ctx *ctx, double *thr_dev, double value);
 size_t vw_sure_workspace(int64_t batch, int64_t n);
 int vw_launch_sure(vw_ctx *ctx, const double *c, int64_t batch, int64_t n, int64_t ld, const double *sigma_dev, void *ws,
                    double *thr_dev, double *risk_dev);

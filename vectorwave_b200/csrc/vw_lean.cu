@@ -6,7 +6,7 @@
 // generic (shared-or-global) store pointers, 64-bit pointer walks, per-level integer divisions, 64-bit tile index
 // arithmetic.  The kernels here take only the case the benchmark configs are made of --
 //   bulk-copy-aligned rows, PERIODIC / ZERO_PADDING / span boundary, compile-time filter length with the taps in uniform
-//   registers (L <= 12, or a quadrature-mirror pair up to 20), full detail mask, no threshold-on-load --
+//   registers (L <= 12, or a quadrature-mirror pair up to 20), full detail mask (the synthesis thresholds W tiles on load) --
 // and spend one integer instruction per shared-memory access: shared memory is addressed by 32-bit element offsets into
 // one `extern __shared__ double[]`, every item is a full item (tile buffers carry slack behind the tile, so items that
 // overshoot the tile end compute on garbage that nothing valid ever reads), per-level geometry comes from the host in

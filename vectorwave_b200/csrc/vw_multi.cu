@@ -139,6 +139,8 @@ struct vw_multi {
     std::vector<cudaEvent_t> ev_t0, ev_t1;   // per device: around the halo copy this device RECEIVES
     std::vector<double *> msg_send, msg_recv;   // synthesis halo messages (device memory, grow-only)
     std::vector<size_t> msg_cap;
+    std::vector<char *> den_buf;   // vw_swt_denoise_sharded per device: threshold, median state and histograms (grow-only)
+    std::vector<size_t> den_cap;
     std::string err;
 };
 
@@ -286,10 +288,14 @@ int vw_span_unpack_inverse(vw_ctx *ctx, const vw_span_plan *plan, const double *
     return finish(ctx, flags | VW_FLAG_NO_SYNC, false);
 }
 
-int vw_modwt_inverse_span_all(vw_ctx *ctx, const vw_span_plan *plan, const double *w, int64_t row_stride, const double *v,
-                              const double *hs, const double *gs, int32_t order, double *xout, uint32_t flags) {
+}  // extern "C"
+
+// thr_dev == nullptr: the plain synthesis; otherwise one threshold applied to every W sample as the kernels load it
+static int inverse_span_all(vw_ctx *ctx, const vw_span_plan *plan, const double *w, int64_t row_stride, const double *v,
+                            const double *hs, const double *gs, int32_t order, const double *thr_dev, int32_t soft, double *xout,
+                            uint32_t flags, const char *name) {
     if (!ctx) return VW_ENULL;
-    DeviceGuard g(ctx, "vw_modwt_inverse_span_all");
+    DeviceGuard g(ctx, name);
     int rc;
     if ((rc = check_plan(ctx, plan))) return rc;
     if (!(flags & VW_FLAG_DEVICE_PTRS)) return vw_fail(ctx, VW_EUNSUPPORTED, "span calls take device pointers only");
@@ -313,12 +319,29 @@ int vw_modwt_inverse_span_all(vw_ctx *ctx, const vw_span_plan *plan, const doubl
             }
             dst = work[cur];
         }
-        rc = vw_modwt_inverse_span(ctx, vext, w + (int64_t)(p.first_i[gi] - 1) * row_stride + p.lead_w, row_stride, s_in - s_out,
-                                   n + s_out, hs, gs, p.l, p.first_i[gi], p.nlev_i[gi], order, dst, fl);
+        rc = inverse_span_device(ctx, vext, w + (int64_t)(p.first_i[gi] - 1) * row_stride + p.lead_w, row_stride, s_in - s_out,
+                                 n + s_out, hs, gs, p.l, p.first_i[gi], p.nlev_i[gi], order, dst, fl, thr_dev, soft);
         if (rc) return rc;
         if (gi > 0) { vext = work[cur]; cur ^= 1; }
     }
     return finish(ctx, flags, false);
+}
+
+extern "C" {
+
+int vw_modwt_inverse_span_all(vw_ctx *ctx, const vw_span_plan *plan, const double *w, int64_t row_stride, const double *v,
+                              const double *hs, const double *gs, int32_t order, double *xout, uint32_t flags) {
+    return inverse_span_all(ctx, plan, w, row_stride, v, hs, gs, order, nullptr, 0, xout, flags, "vw_modwt_inverse_span_all");
+}
+
+int vw_modwt_inverse_span_all_thr(vw_ctx *ctx, const vw_span_plan *plan, const double *w, int64_t row_stride, const double *v,
+                                  const double *hs, const double *gs, int32_t order, const double *thr_dev, int32_t soft,
+                                  double *xout, uint32_t flags) {
+    if (ctx && !thr_dev) {
+        DeviceGuard g(ctx, "vw_modwt_inverse_span_all_thr");
+        return vw_fail(ctx, VW_ENULL, "threshold pointer cannot be null");
+    }
+    return inverse_span_all(ctx, plan, w, row_stride, v, hs, gs, order, thr_dev, soft, xout, flags, "vw_modwt_inverse_span_all_thr");
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -351,6 +374,7 @@ int vw_init_multi(const int *devices, int32_t ndev, vw_multi **out) {
             cudaEventCreate(&e2) != cudaSuccess) { vw_destroy_multi(m); return VW_ECUDA; }
         m->ev_ready.push_back(e0); m->ev_t0.push_back(e1); m->ev_t1.push_back(e2);
         m->msg_send.push_back(nullptr); m->msg_recv.push_back(nullptr); m->msg_cap.push_back(0);
+        m->den_buf.push_back(nullptr); m->den_cap.push_back(0);
         // peer access to both ring neighbours (NVLink through NVSwitch on the box; cudaMemcpyPeerAsync falls back to a
         // staged copy where access cannot be enabled, so a refusal is not fatal)
         for (int nb : {(r + 1) % ndev, (r + ndev - 1) % ndev}) {
@@ -385,6 +409,7 @@ int vw_destroy_multi(vw_multi *m) {
             cudaStreamSynchronize(m->ctx[r]->stream);
             if (r < m->ev_ready.size()) { cudaEventDestroy(m->ev_ready[r]); cudaEventDestroy(m->ev_t0[r]); cudaEventDestroy(m->ev_t1[r]); }
             if (r < m->msg_send.size()) { if (m->msg_send[r]) cudaFree(m->msg_send[r]); if (m->msg_recv[r]) cudaFree(m->msg_recv[r]); }
+            if (r < m->den_buf.size() && m->den_buf[r]) cudaFree(m->den_buf[r]);
         }
         vw_destroy(m->ctx[r]);
     }
@@ -473,9 +498,12 @@ int vw_modwt_forward_sharded(vw_multi *m, const vw_span_plan *plan, double *cons
     return VW_OK;
 }
 
-int vw_modwt_inverse_sharded(vw_multi *m, const vw_span_plan *plan, double *const *w, int64_t row_stride, double *const *v,
-                             const double *hs, const double *gs, int32_t mode, int32_t order, double *const *xout,
-                             float *exchange_ms, uint32_t flags) {
+}  // extern "C"
+
+// thr == nullptr: the plain synthesis; else thr[r] is device r's threshold, applied to W on load (vw_modwt_inverse_span_all_thr)
+static int inverse_sharded(vw_multi *m, const vw_span_plan *plan, double *const *w, int64_t row_stride, double *const *v,
+                           const double *hs, const double *gs, int32_t mode, int32_t order, double *const *xout,
+                           float *exchange_ms, uint32_t flags, const double *const *thr, int32_t soft) {
     int rc;
     if ((rc = multi_check(m, plan, mode))) return rc;
     if (!xout || !w || !v) return multi_fail(m, VW_ENULL, "per-device pointer arrays cannot be null");
@@ -519,7 +547,10 @@ int vw_modwt_inverse_sharded(vw_multi *m, const vw_span_plan *plan, double *cons
     {
         std::vector<int> rcs;
         const uint32_t fl = (flags & ~VW_FLAG_CHECK_FINITE) | VW_FLAG_DEVICE_PTRS | VW_FLAG_NO_SYNC;
-        run_on_all_devices(m, [&](int r) { return vw_modwt_inverse_span_all(m->ctx[r], plan, w[r], row_stride, v[r], hs, gs, order, xout[r], fl); }, rcs);
+        run_on_all_devices(m, [&](int r) {
+            return thr ? vw_modwt_inverse_span_all_thr(m->ctx[r], plan, w[r], row_stride, v[r], hs, gs, order, thr[r], soft, xout[r], fl)
+                       : vw_modwt_inverse_span_all(m->ctx[r], plan, w[r], row_stride, v[r], hs, gs, order, xout[r], fl);
+        }, rcs);
         for (int r = 0; r < P; r++) if ((rc = multi_from_ctx(m, r, rcs[r]))) return rc;
     }
     // msg_send of rank r is read by rank r-1's stream: the next pack on r must not overwrite it early.  Both streams are
@@ -538,6 +569,127 @@ int vw_modwt_inverse_sharded(vw_multi *m, const vw_span_plan *plan, double *cons
         DeviceGuard g(m->ctx[r]->device);
         cudaStreamWaitEvent(m->ctx[r]->stream, m->ev_ready[left], 0);
     }
+    return VW_OK;
+}
+
+extern "C" {
+
+int vw_modwt_inverse_sharded(vw_multi *m, const vw_span_plan *plan, double *const *w, int64_t row_stride, double *const *v,
+                             const double *hs, const double *gs, int32_t mode, int32_t order, double *const *xout,
+                             float *exchange_ms, uint32_t flags) {
+    return inverse_sharded(m, plan, w, row_stride, v, hs, gs, mode, order, xout, exchange_ms, flags, nullptr, 0);
+}
+
+// One long signal denoised across the devices: analysis, the exact median of |W_1| over the whole signal, synthesis with
+// the threshold applied on load.  The median runs select_median's seven rounds with the histograms reduced ON the
+// devices: after each rank's histogram every device pulls the others' tables (cudaMemcpyPeerAsync, ordered by the
+// ranks' events) and sums them itself, so all devices pick from the same sum with no host round trip between rounds.
+// Each round's own table has its own slot, so a table is never rewritten while a peer may still be reading it.
+int vw_swt_denoise_sharded(vw_multi *m, const vw_span_plan *plan, double *const *xext, const double *hs, const double *gs,
+                           int32_t mode, int32_t order, double threshold, int32_t soft, double *const *w, int64_t row_stride,
+                           double *const *v, double *const *xout, double *threshold_out, uint32_t flags) {
+    int rc;
+    if ((rc = multi_check(m, plan, mode))) return rc;
+    if (!xext || !w || !v || !xout) return multi_fail(m, VW_ENULL, "per-device pointer arrays cannot be null");
+    const int P = (int)m->ctx.size();
+    const vw_span_plan &p = *plan;
+    for (int r = 0; r < P; r++)
+        if (!xext[r] || !w[r] || !v[r] || !xout[r]) return multi_fail(m, VW_ENULL, "a per-device buffer is null");
+    if (order != VW_ORDER_SPLIT && order != VW_ORDER_PAIR) return multi_fail(m, VW_EINVAL, "unknown synthesis order " + std::to_string(order));
+    if (p.ngroups_f < 1 || p.ngroups_i < 1 || p.n_local < 1) return multi_fail(m, VW_EINVAL, "span plan is not initialised (vw_span_plan_query)");
+    const int64_t n = p.n_local, n_total = n * (int64_t)P;
+    // 0. every span is checked before anything is computed (nothing is written to xout on failure)
+    if (flags & VW_FLAG_CHECK_FINITE)
+        for (int r = 0; r < P; r++) {
+            vw_ctx *c = m->ctx[r];
+            DeviceGuard g(c, "vw_swt_denoise_sharded");
+            if ((rc = check_finite(c, xext[r] + p.lead, 1, n, n, "signal")))
+                return multi_fail(m, rc, "rank " + std::to_string(r) + " (device " + std::to_string(c->device) + "): " + vw_last_error(c));
+        }
+    const uint32_t fl = (flags & ~VW_FLAG_CHECK_FINITE) | VW_FLAG_NO_SYNC;
+    // 1. analysis
+    if ((rc = vw_modwt_forward_sharded(m, plan, xext, hs, gs, mode, w, row_stride, v, nullptr, fl))) return rc;
+    // 2. per-device work space: [threshold | summed table | one own table per round | the ranks' tables | median state]
+    constexpr int kEntries = 2 << 12;   // the largest round's table (vw_span_median_bins)
+    const size_t tab = (size_t)kEntries * 8;
+    const size_t off_sum = 256, off_own = off_sum + tab, off_gather = off_own + VW_SPAN_MEDIAN_ROUNDS * tab,
+                 off_state = off_gather + (size_t)P * tab;
+    const size_t need = off_state + vw_span_median_state_bytes(n);
+    bool grow = false;
+    for (int r = 0; r < P; r++) grow = grow || m->den_cap[r] < need;
+    // a peer may still be reading an earlier call's tables from its own stream: every device drains before any regrowth
+    if (grow && (rc = vw_multi_synchronize(m))) return rc;
+    for (int r = 0; r < P; r++) {
+        vw_ctx *c = m->ctx[r];
+        if (m->den_cap[r] >= need) continue;
+        DeviceGuard g(c, "vw_swt_denoise_sharded");
+        if (m->den_buf[r]) cudaFree(m->den_buf[r]);
+        m->den_buf[r] = nullptr; m->den_cap[r] = 0;
+        if ((rc = multi_from_ctx(m, r, vw_cuda_check(c, cudaMalloc((void **)&m->den_buf[r], need), "denoise work space")))) return rc;
+        m->den_cap[r] = need;
+    }
+    std::vector<double *> thr(P);
+    for (int r = 0; r < P; r++) thr[r] = (double *)m->den_buf[r];
+    // 3. the threshold: the same value on every device
+    if (threshold < 0) {
+        auto at = [&](int r, size_t off) { return m->den_buf[r] + off; };
+        for (int r = 0; r < P; r++)
+            if ((rc = multi_from_ctx(m, r, vw_span_median_init(m->ctx[r], at(r, off_state), n_total)))) return rc;
+        for (int round = 0; round < VW_SPAN_MEDIAN_ROUNDS; round++) {
+            const int entries = vw_span_median_bins(round);
+            for (int r = 0; r < P; r++) {
+                vw_ctx *c = m->ctx[r];
+                uint64_t *own = (uint64_t *)(at(r, off_own) + (size_t)round * tab);
+                if ((rc = multi_from_ctx(m, r, vw_span_median_hist(c, at(r, off_state), w[r] + p.lead_w, n, round, own)))) return rc;
+                DeviceGuard g(c->device);
+                if ((rc = multi_from_ctx(m, r, vw_cuda_check(c, cudaEventRecord(m->ev_ready[r], c->stream), "event record")))) return rc;
+            }
+            for (int r = 0; r < P; r++) {
+                vw_ctx *c = m->ctx[r];
+                uint64_t *gather = (uint64_t *)at(r, off_gather);
+                {
+                    DeviceGuard g(c->device);
+                    for (int q = 0; q < P; q++) {
+                        if (q == r) continue;
+                        cudaError_t e = cudaStreamWaitEvent(c->stream, m->ev_ready[q], 0);
+                        if (e == cudaSuccess)
+                            e = cudaMemcpyPeerAsync(gather + (size_t)q * entries, c->device, at(q, off_own) + (size_t)round * tab,
+                                                    m->ctx[q]->device, (size_t)entries * 8, c->stream);
+                        if ((rc = multi_from_ctx(m, r, vw_cuda_check(c, e, "median histogram exchange")))) return rc;
+                    }
+                }
+                uint64_t *sum = (uint64_t *)at(r, off_sum);
+                {
+                    DeviceGuard g(c, "vw_swt_denoise_sharded");
+                    rc = vw_launch_span_hist_sum(c, gather, (const uint64_t *)(at(r, off_own) + (size_t)round * tab), P, r, entries, sum);
+                }
+                if ((rc = multi_from_ctx(m, r, rc))) return rc;
+                if ((rc = multi_from_ctx(m, r, vw_span_median_pick(c, at(r, off_state), round, sum)))) return rc;
+            }
+        }
+        const double factor = sqrt(2.0 * log((double)n_total));   // k_select_finish's factor, from the total length
+        for (int r = 0; r < P; r++)
+            if ((rc = multi_from_ctx(m, r, vw_span_median_value(m->ctx[r], at(r, off_state), factor, thr[r])))) return rc;
+    } else {
+        for (int r = 0; r < P; r++) {
+            DeviceGuard g(m->ctx[r], "vw_swt_denoise_sharded");
+            if ((rc = multi_from_ctx(m, r, vw_launch_span_fixed(m->ctx[r], thr[r], threshold)))) return rc;
+        }
+    }
+    // 4. the synthesis exchange and the thresholded cascades
+    if ((rc = inverse_sharded(m, plan, w, row_stride, v, hs, gs, mode, order, xout, nullptr, fl, thr.data(), soft))) return rc;
+    if (threshold_out) {
+        if (threshold < 0) {
+            vw_ctx *c = m->ctx[0];
+            DeviceGuard g(c->device);
+            if ((rc = multi_from_ctx(m, 0, vw_cuda_check(c, cudaMemcpyAsync(threshold_out, thr[0], 8, cudaMemcpyDeviceToHost, c->stream), "small copy"))))
+                return rc;
+            if ((rc = multi_from_ctx(m, 0, vw_cuda_check(c, cudaStreamSynchronize(c->stream), "threshold copy")))) return rc;
+        } else {
+            *threshold_out = threshold;
+        }
+    }
+    if (!(flags & VW_FLAG_NO_SYNC)) return vw_multi_synchronize(m);
     return VW_OK;
 }
 

@@ -218,6 +218,232 @@ static int select_median(vw_ctx *ctx, const double *w1, int64_t batch, int64_t n
     return vw_cuda_check(ctx, cudaGetLastError(), "universal threshold launch");
 }
 
+// ---- the same selection over a signal split into spans on several ranks -------------------------------------------
+// select_median's seven digit rounds with the histogram handed out between "histogram" and "pick": every rank counts
+// its own span into a u64 table, the caller sums the tables over the ranks, and every rank picks from the identical sum,
+// so the decided prefixes and remaining ranks stay identical everywhere.  The candidate buffer of round 2 is rank-local:
+// a rank whose bucket overflows it (a constant span) keeps histogramming its full span, the others their candidates,
+// and the sum is the same exact count either way.
+namespace {
+struct SpanSel {             // device state blob: SelState first (the per-row kernels above run on it with batch 1)
+    SelState s;
+    long long n_total;
+    long long pad[3];
+};
+static_assert(sizeof(SpanSel) <= 256, "span selection state fits its 256-byte header");
+
+constexpr int kSpanRounds = VW_SPAN_MEDIAN_ROUNDS;
+int span_bits(int round) { return round < 2 ? kBig : 8; }
+int span_shift(int round) { return round < 2 ? 64 - kBig * (round + 1) : 64 - 2 * kBig - 8 * (round - 1); }
+unsigned int span_cap(int64_t n_local) {
+    int64_t cap64 = n_local / 64;
+    if (cap64 < 1024) cap64 = 1024;
+    if (cap64 > (1 << 20)) cap64 = 1 << 20;
+    return (unsigned int)cap64;
+}
+
+__global__ void k_span_init(SpanSel *st, long long n_total) {
+    st->s.prefix[0] = st->s.prefix[1] = 0ull;
+    st->s.rank[1] = (unsigned long long)(n_total / 2);
+    st->s.rank[0] = (n_total % 2 == 0) ? (unsigned long long)(n_total / 2 - 1) : (unsigned long long)(n_total / 2);
+    st->s.count[0] = st->s.count[1] = 0u;
+    st->n_total = n_total;
+}
+
+// k_select_hist on one span, accumulated into a u64 table [2][1 << BITS] (the sum over ranks may exceed 2^32)
+template <int BITS>
+__global__ void __launch_bounds__(256)
+k_span_hist(const double *__restrict__ w, int64_t n, const SpanSel *__restrict__ st, int shift,
+            unsigned long long *__restrict__ hist, const double *__restrict__ cand, unsigned int cap) {
+    constexpr int BINS = 1 << BITS;
+    __shared__ unsigned int sh[2][BINS];
+    for (int i = threadIdx.x; i < 2 * BINS; i += blockDim.x) (&sh[0][0])[i] = 0;
+    __syncthreads();
+    const unsigned long long p0 = st->s.prefix[0], p1 = st->s.prefix[1];
+    const bool same = p0 == p1;
+    const int hs = shift + BITS;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x, t0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool use_cand = cand != nullptr && st->s.count[0] <= cap && st->s.count[1] <= cap;
+    if (!use_cand) {
+        for (int64_t t = t0; t < n; t += stride) {
+            const unsigned long long key = key_of(w[t]);
+            const unsigned long long hi = hs >= 64 ? 0ull : (key >> hs);
+            const unsigned int dg = (unsigned int)(key >> shift) & (BINS - 1);
+            if (hi == p0) atomicAdd(&sh[0][dg], 1u);
+            if (!same && hi == p1) atomicAdd(&sh[1][dg], 1u);
+        }
+    } else {
+        for (int which = 0; which < (same ? 1 : 2); which++) {
+            const double *src = cand + (size_t)which * cap;
+            const unsigned long long pw = which ? p1 : p0;
+            const int64_t len = st->s.count[which];
+            for (int64_t t = t0; t < len; t += stride) {
+                const unsigned long long key = key_of(src[t]);
+                const unsigned long long hi = hs >= 64 ? 0ull : (key >> hs);
+                if (hi == pw) atomicAdd(&sh[which][(unsigned int)(key >> shift) & (BINS - 1)], 1u);
+            }
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < BINS; i += blockDim.x) {
+        const unsigned int c0 = sh[0][i], c1 = same ? c0 : sh[1][i];
+        if (c0) atomicAdd(&hist[i], (unsigned long long)c0);
+        if (c1) atomicAdd(&hist[BINS + i], (unsigned long long)c1);
+    }
+}
+
+// k_select_pick on a summed u64 table (left as it is: it belongs to the caller); one block per tracked rank
+template <int BITS>
+__global__ void __launch_bounds__(256) k_span_pick(SpanSel *st, const unsigned long long *__restrict__ hist) {
+    constexpr int BINS = 1 << BITS, PER = BINS / 256 > 0 ? BINS / 256 : 1;
+    __shared__ unsigned long long part[256];
+    const int which = (int)blockIdx.x;
+    const unsigned long long *h = hist + (size_t)which * BINS;
+    const int tid = threadIdx.x;
+    unsigned long long mine = 0;
+    unsigned long long loc[PER];
+#pragma unroll
+    for (int q = 0; q < PER; q++) { const int bin = tid * PER + q; loc[q] = bin < BINS ? h[bin] : 0ull; mine += loc[q]; }
+    part[tid] = mine;
+    __syncthreads();
+    if (tid == 0) {
+        unsigned long long run = 0;
+        for (int q = 0; q < 256; q++) { const unsigned long long c = part[q]; part[q] = run; run += c; }
+    }
+    __syncthreads();
+    const unsigned long long r = st->s.rank[which];
+    unsigned long long cum = part[tid];
+    __syncthreads();
+    if (r >= cum && r < cum + mine) {
+#pragma unroll
+        for (int q = 0; q < PER; q++) {
+            if (r < cum + loc[q]) {
+                st->s.rank[which] = r - cum;
+                st->s.prefix[which] = (st->s.prefix[which] << BITS) | (unsigned long long)(tid * PER + q);
+                break;
+            }
+            cum += loc[q];
+        }
+    }
+}
+
+// k_select_finish with the total length from the state
+__global__ void k_span_finish(const SpanSel *st, double factor, double *thr) {
+    const double lo = __longlong_as_double((long long)st->s.prefix[0]);
+    const double hi = __longlong_as_double((long long)st->s.prefix[1]);
+    const double med = (st->n_total % 2 == 0) ? __ddiv_rn(__dadd_rn(lo, hi), 2.0) : hi;
+    *thr = factor >= 0.0 ? __dmul_rn(__ddiv_rn(med, 0.6745), factor) : med;
+}
+
+// out[i] = own[i] + sum over the other ranks' tables (gather[q], q != self), in rank order
+__global__ void __launch_bounds__(256) k_span_hist_sum(const unsigned long long *__restrict__ gather,
+                                                       const unsigned long long *__restrict__ own, int ranks, int self,
+                                                       int entries, unsigned long long *__restrict__ out) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < entries; i += gridDim.x * blockDim.x) {
+        unsigned long long s = 0;
+        for (int q = 0; q < ranks; q++) s += q == self ? own[i] : gather[(size_t)q * entries + i];
+        out[i] = s;
+    }
+}
+
+__global__ void k_span_fixed(double *thr, double value) { *thr = value; }
+}  // namespace
+
+static int vw_span_rounds_check(vw_ctx *ctx, int32_t round) {
+    if (round < 0 || round >= kSpanRounds) return vw_fail(ctx, VW_EINVAL, "median round %d outside 0..%d", round, kSpanRounds - 1);
+    return VW_OK;
+}
+
+int vw_launch_span_hist_sum(vw_ctx *ctx, const uint64_t *gather, const uint64_t *own, int ranks, int self, int entries,
+                            uint64_t *out) {
+    k_span_hist_sum<<<(entries + 255) / 256, 256, 0, ctx->stream>>>((const unsigned long long *)gather, (const unsigned long long *)own,
+                                                                     ranks, self, entries, (unsigned long long *)out);
+    ctx->launches++;
+    return vw_cuda_check(ctx, cudaGetLastError(), "median histogram sum launch");
+}
+
+int vw_launch_span_fixed(vw_ctx *ctx, double *thr_dev, double value) {
+    k_span_fixed<<<1, 1, 0, ctx->stream>>>(thr_dev, value);
+    ctx->launches++;
+    return vw_cuda_check(ctx, cudaGetLastError(), "threshold store launch");
+}
+
+extern "C" {
+
+int32_t vw_span_median_bins(int32_t round) {
+    if (round < 0 || round >= kSpanRounds) return 0;
+    return 2 << span_bits(round);
+}
+
+size_t vw_span_median_state_bytes(int64_t n_local) {
+    if (n_local < 1) return 0;
+    return 256 + (size_t)2 * span_cap(n_local) * sizeof(double);
+}
+
+int vw_span_median_init(vw_ctx *ctx, void *state, int64_t n_total) {
+    if (!ctx) return VW_ENULL;
+    vwshim::DeviceGuard g(ctx, "vw_span_median_init");
+    if (!state) return vw_fail(ctx, VW_ENULL, "median state cannot be null");
+    if (n_total < 1) return vw_fail(ctx, VW_EEMPTY, "signal cannot be empty");
+    k_span_init<<<1, 1, 0, ctx->stream>>>((SpanSel *)state, (long long)n_total);
+    ctx->launches++;
+    return vw_cuda_check(ctx, cudaGetLastError(), "median init launch");
+}
+
+int vw_span_median_hist(vw_ctx *ctx, void *state, const double *c, int64_t n_local, int32_t round, uint64_t *hist) {
+    if (!ctx) return VW_ENULL;
+    vwshim::DeviceGuard g(ctx, "vw_span_median_hist");
+    int rc;
+    if ((rc = vw_span_rounds_check(ctx, round))) return rc;
+    if (!state || !c || !hist) return vw_fail(ctx, VW_ENULL, "median buffers cannot be null");
+    if (n_local < 1) return vw_fail(ctx, VW_EEMPTY, "span cannot be empty");
+    SpanSel *st = (SpanSel *)state;
+    const unsigned int cap = span_cap(n_local);
+    double *cand = (double *)((char *)state + 256);
+    const int bits = span_bits(round), shift = span_shift(round);
+    if ((rc = vw_cuda_check(ctx, cudaMemsetAsync(hist, 0, (size_t)(2 << bits) * sizeof(uint64_t), ctx->stream), "median memset")))
+        return rc;
+    int64_t chunks = (n_local + 256 * 16 - 1) / (256 * 16);
+    if (chunks > (int64_t)ctx->sm_count * 16) chunks = (int64_t)ctx->sm_count * 16;
+    if (chunks < 1) chunks = 1;
+    if (round == 2) {
+        // the 24 decided bits are the same on every rank: compact this span's keys that share them
+        const dim3 grid((unsigned)chunks, 1, 1);
+        k_select_collect<<<grid, 256, 0, ctx->stream>>>(c, 1, n_local, n_local, &st->s, 2 * kBig, cand, cap);
+        k_select_mirror_count<<<1, 128, 0, ctx->stream>>>(&st->s, 1);
+        ctx->launches += 2;
+    }
+    unsigned long long *h = (unsigned long long *)hist;
+    if (bits == kBig) k_span_hist<kBig><<<(unsigned)chunks, 256, 0, ctx->stream>>>(c, n_local, st, shift, h, nullptr, 0u);
+    else k_span_hist<8><<<(unsigned)chunks, 256, 0, ctx->stream>>>(c, n_local, st, shift, h, cand, cap);
+    ctx->launches++;
+    return vw_cuda_check(ctx, cudaGetLastError(), "median histogram launch");
+}
+
+int vw_span_median_pick(vw_ctx *ctx, void *state, int32_t round, const uint64_t *hist_sum) {
+    if (!ctx) return VW_ENULL;
+    vwshim::DeviceGuard g(ctx, "vw_span_median_pick");
+    int rc;
+    if ((rc = vw_span_rounds_check(ctx, round))) return rc;
+    if (!state || !hist_sum) return vw_fail(ctx, VW_ENULL, "median buffers cannot be null");
+    const unsigned long long *h = (const unsigned long long *)hist_sum;
+    if (span_bits(round) == kBig) k_span_pick<kBig><<<2, 256, 0, ctx->stream>>>((SpanSel *)state, h);
+    else k_span_pick<8><<<2, 256, 0, ctx->stream>>>((SpanSel *)state, h);
+    ctx->launches++;
+    return vw_cuda_check(ctx, cudaGetLastError(), "median pick launch");
+}
+
+int vw_span_median_value(vw_ctx *ctx, const void *state, double factor, double *out_dev) {
+    if (!ctx) return VW_ENULL;
+    vwshim::DeviceGuard g(ctx, "vw_span_median_value");
+    if (!state || !out_dev) return vw_fail(ctx, VW_ENULL, "median buffers cannot be null");
+    k_span_finish<<<1, 1, 0, ctx->stream>>>((const SpanSel *)state, factor, out_dev);
+    ctx->launches++;
+    return vw_cuda_check(ctx, cudaGetLastError(), "median value launch");
+}
+
+}  // extern "C"
+
 // ---- SURE threshold (CORE/denoising/WaveletDenoiser.java:441-492) -------------------------------------------------
 // The reference scores every candidate threshold t = |c_i| with a full pass over the coefficients (an O(n^2) double
 // loop) and keeps the first minimum in ascending order of t.  Here one thread owns kSureCand candidates and walks the

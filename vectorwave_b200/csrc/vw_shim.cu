@@ -1541,6 +1541,19 @@ int vw_modwt_stream_level(vw_ctx *ctx, const double *vin, int64_t batch, int64_t
 int vw_modwt_inverse_span(vw_ctx *ctx, const double *vin, const double *w, int64_t level_stride_w, int64_t halo,
                           int64_t n_local, const double *hs, const double *gs, int32_t l, int32_t first_level,
                           int32_t nlevels, int32_t order, double *vout, uint32_t flags) {
+    return vwshim::inverse_span_device(ctx, vin, w, level_stride_w, halo, n_local, hs, gs, l, first_level, nlevels, order, vout,
+                                       flags, nullptr, 0);
+}
+
+}  // extern "C"
+
+namespace vwshim {
+// vw_modwt_inverse_span, optionally with one threshold (device scalar) applied to every W sample the group reads, halo
+// included: the tile, column and column-pair kernels threshold on load; the per-level kernels have no such form, so each
+// level's W row is thresholded into a scratch copy first (the caller's W stays as it is)
+int inverse_span_device(vw_ctx *ctx, const double *vin, const double *w, int64_t level_stride_w, int64_t halo, int64_t n_local,
+                        const double *hs, const double *gs, int32_t l, int32_t first_level, int32_t nlevels, int32_t order,
+                        double *vout, uint32_t flags, const double *thr_dev, int32_t thr_soft) {
     if (!ctx) return VW_ENULL;
     DeviceGuard g(ctx, "vw_modwt_inverse_span");
     ctx->plan_lean_ok = true;
@@ -1560,12 +1573,12 @@ int vw_modwt_inverse_span(vw_ctx *ctx, const double *vin, const double *w, int64
     const bool column_first = nlevels == 1 && first_level >= vw_column_min_level(ctx, l, false) && ctx->opt_poly != 0;
     if (!exact && !(flags & VW_FLAG_NO_FUSE) && nlevels == 2 && first_level >= vw_column_min_level(ctx, l, false) && ctx->opt_poly != 0) {
         rc = vw_column_synthesis2(ctx, vin, 0, w + level_stride_w, 0, w, 0, vout, 0, n_in, 0, n_local, 1, f, l,
-                                  (int64_t)1 << (first_level - 1), VW_MODE_LINEAR, nullptr, 0, 0, 0);
+                                  (int64_t)1 << (first_level - 1), VW_MODE_LINEAR, thr_dev, 0, thr_soft, 0);
         if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
     }
     if (rc == VW_EUNSUPPORTED && !exact && !(flags & VW_FLAG_NO_FUSE) && !column_first) {
         VwFusedInv p{vin, n_in, w, n_in, level_stride_w, nlevels >= 64 ? ~0ull : ((1ull << nlevels) - 1), vout, n_local,
-                     1, n_in, n_local, l, first_level, nlevels, VW_MODE_LINEAR, nullptr, 0, 0, 0};
+                     1, n_in, n_local, l, first_level, nlevels, VW_MODE_LINEAR, thr_dev, 0, thr_soft, 0};
         rc = vw_fused_inverse(ctx, p, f);
         if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
     }
@@ -1585,17 +1598,27 @@ int vw_modwt_inverse_span(vw_ctx *ctx, const double *vin, const double *w, int64
             }
             rc = VW_EUNSUPPORTED;
             if (nlevels == 1 && !exact && !(flags & VW_FLAG_NO_FUSE) && d >= ((int64_t)1 << (vw_column_min_level(ctx, l, false) - 1)) && ctx->opt_poly != 0) {
-                rc = vw_column_synthesis(ctx, cur, 0, w, 0, dst, 0, n_in, 0, n_out, 1, f, l, d, VW_MODE_LINEAR, default_align());
+                rc = vw_column_synthesis(ctx, cur, 0, w, 0, dst, 0, n_in, 0, n_out, 1, f, l, d, VW_MODE_LINEAR, default_align(), thr_dev,
+                                         0, thr_soft);
                 if (rc != VW_OK && rc != VW_EUNSUPPORTED) return rc;
             }
-            if (rc == VW_EUNSUPPORTED)
-                rc = vw_launch_synthesis_level(ctx, cur, 0, w + (int64_t)i * level_stride_w, 0, dst, 0, n_in, 0, n_out, 1, f, l, d,
-                                               VW_MODE_LINEAR, default_align(), order == VW_ORDER_PAIR, exact);
+            if (rc == VW_EUNSUPPORTED) {
+                const double *wj = w + (int64_t)i * level_stride_w;
+                if (thr_dev) {
+                    void *p;
+                    if ((rc = vw_scratch(ctx, 4, (size_t)n_in * 8, &p))) return rc;
+                    if ((rc = vw_cuda_check(ctx, cudaMemcpyAsync(p, wj, (size_t)n_in * 8, cudaMemcpyDeviceToDevice, ctx->stream), "d2d")))
+                        return rc;
+                    if ((rc = vw_launch_threshold(ctx, (double *)p, 1, n_in, n_in, thr_dev, 0, thr_soft))) return rc;
+                    wj = (const double *)p;
+                }
+                rc = vw_launch_synthesis_level(ctx, cur, 0, wj, 0, dst, 0, n_in, 0, n_out, 1, f, l, d, VW_MODE_LINEAR, default_align(),
+                                               order == VW_ORDER_PAIR, exact);
+            }
             if (rc) return rc;
             cur = dst;
         }
     }
     return finish(ctx, flags, false);
 }
-
-}  // extern "C"
+}  // namespace vwshim

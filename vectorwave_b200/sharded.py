@@ -23,8 +23,8 @@ import torch
 import torch.distributed as dist
 
 from . import _native
-from ._native import Engine, ORDER_SPLIT
-from .errors import IllegalArgumentException
+from ._native import Engine, ORDER_PAIR, ORDER_SPLIT, SPAN_MEDIAN_ROUNDS, span_median_bins
+from .errors import ErrorCode, IllegalArgumentException, InvalidSignalException
 from .wavelets import BoundaryMode
 
 SCALE = 1.0 / math.sqrt(2.0)
@@ -323,3 +323,47 @@ class SpanShardedMODWT:
             vext = work[cur]
             cur ^= 1
         return out
+
+    # -- SWT denoise of the whole signal ----------------------------------------------------------------------
+    def denoise(self, x_local, threshold=-1.0, soft=True):
+        """VectorWaveSwtAdapter.denoise of the whole signal (vw_swt_denoise with batch = 1 on all world * n_local samples),
+        computed span by span: decompose, threshold every detail level, reconstruct.  threshold < 0: the universal
+        threshold median(|W_1|) / 0.6745 * sqrt(2 ln N) with the exact median over every rank's W_1 (seven histogram
+        rounds, one all_reduce(SUM) of an int64 table per round over this object's group); otherwise the given value.
+        V_J is not thresholded.  Returns (this rank's denoised span, the threshold).  Every rank must call it.  Needs the
+        default (plan) schedule."""
+        if self.plan is None:
+            raise IllegalArgumentException("denoise needs the default schedule (engine launch groups, up-front halo exchange)")
+        n, dev = self.n_local, x_local.device
+        if x_local.numel() != n:
+            raise IllegalArgumentException(f"expected a span of {n} samples, got {x_local.numel()}")
+        # collective validation: every rank reaches the same decision before any other collective, so a NaN on one rank
+        # cannot leave the others waiting in an all_reduce
+        bad = torch.tensor([0 if bool(torch.isfinite(x_local).all()) else 1], dtype=torch.int64, device=dev)
+        if self.world > 1:
+            dist.all_reduce(bad, op=dist.ReduceOp.SUM, group=self.group)
+        if int(bad.item()):
+            raise InvalidSignalException(f"{int(bad.item())} rank(s) hold non-finite values (NaN or Infinity)",
+                                         ErrorCode.VAL_NON_FINITE_VALUES)
+        res = self._forward_plan(x_local)
+        eng = self._eng()
+        n_total = n * self.world
+        if threshold < 0:
+            w1 = res.storage[0, self.lead_w:self.lead_w + n]
+            state = eng.span_median_state(n)
+            eng.span_median_init(state, n_total)
+            for rnd in range(SPAN_MEDIAN_ROUNDS):
+                hist = torch.empty(span_median_bins(rnd), dtype=torch.int64, device=dev)
+                eng.span_median_hist(state, w1, rnd, hist)
+                if self.world > 1:
+                    dist.all_reduce(hist, op=dist.ReduceOp.SUM, group=self.group)
+                eng.span_median_pick(state, rnd, hist)
+            thr = torch.empty(1, dtype=torch.float64, device=dev)
+            eng.span_median_value(state, math.sqrt(2.0 * math.log(float(n_total))), thr)
+        else:
+            thr = torch.full((1,), float(threshold), dtype=torch.float64, device=dev)
+        self.exchange_inverse(res)
+        out = torch.empty(n, dtype=torch.float64, device=dev)
+        order = ORDER_PAIR if self.mode == BoundaryMode.ZERO_PADDING else ORDER_SPLIT   # MultiLevelMODWTTransform.reconstruct
+        eng.inverse_span_all_thr(self.plan, res.storage, res.v, self.hrs, self.grs, order, thr, soft, out)
+        return out, float(thr.item())
